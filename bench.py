@@ -17,6 +17,9 @@ stay those of config 2); `--config 3|4|5` prints the full line of that config in
   4  2^20 independent 4 KiB pages, one stream per page, batched API
   5  8 GiB source-code-like corpus as 8 streams x 1 GiB (one stream cannot exceed 2^32 - 1 bytes,
      src/Snappy.jl:21), the SAME 8 streams sharded over 1/2/4/8 GPUs: strong scaling
+`--steps K` is the number of timed steps of every leg: the headline config, the nested ones and both e2e legs.
+`--dump-outputs DIR` (config 2) writes what the last timed step returned to its caller as DIR/<name>.npy, so that two
+builds run with the same arguments (hence the same inputs) can be compared output for output.
 `--impl reference` times the oracle alone (the reference is Julia and cannot run in this image).
 N > 1 (torchrun), config 2: weak scaling -- N streams of 1 GiB, every stream sharded over the N ranks along
 whole-fragment boundaries; sizes by ncclAllGather on the compute stream, fragments stored straight into the owner's
@@ -33,6 +36,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: a benchmark run leaves nothing in it
 
 import numpy as np  # noqa: E402
 
@@ -61,8 +65,16 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="config 2 only: skip the nested legs of configs 3, 4, 5")
-    ap.add_argument("--extra-steps", type=int, default=3, help="timed steps of each nested config leg")
-    return ap.parse_args()
+    ap.add_argument("--extra-steps", type=int, default=None, help="timed steps of each nested config leg "
+                                                                  "(default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="config 2: write the last timed step's outputs to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.extra_steps is None:
+        args.extra_steps = args.steps
+    if args.dump_outputs and (args.config != 2 or args.impl != "b200"):
+        ap.error("--dump-outputs writes the outputs of config 2 of the b200 arm")
+    return args
 
 
 def measured_peak():
@@ -518,6 +530,24 @@ def timed_loop(ctx, steps, warmup, do_c, do_u, after_c=None):
     return tc, tu, rc, ru
 
 
+DUMP_BYTES = 60 * 10 ** 6  # array data of one --dump-outputs run; with the .npy headers it stays under 64 MB
+
+
+def dump_outputs(where, arrays, seed):
+    """Writes every tensor of `arrays` (name -> 1-D tensor) as where/<name>.npy: float32 when its integers fit one
+    exactly (up to 16 bits), float64 otherwise.  Each gets an equal share of DUMP_BYTES; a longer one is replaced by
+    its elements at sorted positions drawn with `seed`, so the same positions of equally long outputs are compared."""
+    import torch
+    os.makedirs(where, exist_ok=True)
+    keep = DUMP_BYTES // (8 * len(arrays))
+    for name, t in arrays.items():
+        if t.numel() > keep:
+            pos = np.sort(np.random.default_rng(seed).integers(0, t.numel(), keep))
+            t = t[torch.from_numpy(pos).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(where, name + ".npy"), a.astype(np.float32 if a.dtype.itemsize <= 2 else np.float64))
+
+
 def traffic_entry(kernel):
     try:
         with open(os.path.join(ROOT, "profiles", "traffic.json")) as f:
@@ -616,8 +646,10 @@ def config2(ctx, nested=False):
         kstat["l"] += device.last_launch_count(1)
         return out
 
-    tc, tu, rc, back = timed_loop(ctx, steps, 0, do_c, do_u_counted, after_c=after_c)
-    clocks = sampler.stop() if (rank == 0 and not nested) else None
+    try:
+        tc, tu, rc, back = timed_loop(ctx, steps, 0, do_c, do_u_counted, after_c=after_c)
+    finally:
+        clocks = sampler.stop() if (rank == 0 and not nested) else None
     kc, ku = kstat["c"] / steps, kstat["u"] / steps
     launches = kstat["l"] * (world if world > 1 else 1)
 
@@ -666,6 +698,11 @@ def config2(ctx, nested=False):
         # bytes this rank's compress kernel produced: its run of every stream
         ratio = csize / n
         my_c_bytes = int(my_n * ratio)
+    if args.dump_outputs and rank == 0 and not nested:
+        # what compress_device / uncompress_device (or the communicator) handed back in the last timed step
+        outs = {"compressed": stream[:csize], "compressed_index": index}
+        outs.update({"uncompressed": back} if world == 1 else {"uncompressed_%d" % s: back[s] for s in range(world)})
+        dump_outputs(args.dump_outputs, outs, args.seed)
 
     total_bytes = n * (world if world > 1 else 1)  # uncompressed bytes all ranks processed per step
     t_step_ms = (tc + tu) / steps
@@ -723,7 +760,7 @@ def config2(ctx, nested=False):
                 dt = float(t[0])
             return dt, c_len
 
-        reps = max(2, min(args.steps, 10))
+        reps = args.steps
         dt, c_len = e2e_run(host_in.data_ptr(), h_out.data_ptr(), h_back.data_ptr(), reps)
         assert torch.equal(h_back, host_in)
         e2e = {"value": en * world / dt / 1e9, "unit": "GB/s", "h2d_bytes_per_step": (en + c_len) * world,
@@ -740,7 +777,7 @@ def config2(ctx, nested=False):
             p_back = np.empty(en, dtype=np.uint8)
             p_out[::4096] = 0
             p_back[::4096] = 0
-        dtp, _ = e2e_run(p_in.ctypes.data, p_out.ctypes.data, p_back.ctypes.data, max(2, min(reps, 4)))
+        dtp, _ = e2e_run(p_in.ctypes.data, p_out.ctypes.data, p_back.ctypes.data, reps)
         assert np.array_equal(p_back, p_in)
         e2e["pageable"] = {"value": en * world / dtp / 1e9, "unit": "GB/s", "ms_per_step": dtp * 1e3,
                            "of_pinned": dt / dtp,
