@@ -1,12 +1,19 @@
 """Fuzz campaign for the kernel sources on the CPU warp (TEST INFRASTRUCTURE; minutes of CPU, not part of pytest).
 
-    python tools/cpu_warp/fuzz.py [seed] [count]
+    python tools/cpu_warp/fuzz.py [seed] [count] [legs]
 
 Generates `count` inputs (small alphabets, periodic data with mutations, runs, dictionary words, concatenations,
 boundary sizes), then runs: the window compress kernel (shared / global tables, rules 0/1/2, three ring sizes), the
 step-wise chain kernel, the indexed decoder, the page kernels, and the index-free parse on the Snappy.jl and Google
-snappy streams of every input.  Any mismatch against the oracle / the sequential walk is printed; exit status 1.
-Last run (seed 12345, 201 inputs, ~15 min on 8 cores): no mismatch anywhere."""
+snappy streams of every input.  Then the corruption corpus's mutations (tests/test_decode_corruption.py: random and
+boundary faults, truncations, header lies, two faults, accepted quirks) of the multi-fragment streams (Snappy.jl's and
+Google snappy's in turn) go through the index-free decode chain (run_decode_parsed.cpp: parse, tiles, bounded serial
+walk; parse chunks of 512 B, 1 KiB and 4 KiB, and without clean cuts) and the page decoder, against the oracle's status
+and bytes.  `legs`: comma-separated subset of "compress,decode,pages,parse,corrupt" (default: all).  Any mismatch
+against the oracle / the sequential walk is printed; exit status 1.
+Last run of every leg but "corrupt" (seed 12345, 201 inputs, ~15 min on 8 cores): no mismatch anywhere.
+Last run of "corrupt" (seed 12345, 201 inputs: 5028 mutated streams, ~5 min on 8 cores): no mismatch anywhere."""
+import concurrent.futures
 import os
 import subprocess
 import sys
@@ -66,14 +73,16 @@ def main():
     import pyoracle
     seed = int(sys.argv[1]) if len(sys.argv) > 1 else 12345
     count = int(sys.argv[2]) if len(sys.argv) > 2 else 201
+    legs = set(sys.argv[3].split(",")) if len(sys.argv) > 3 else {"compress", "decode", "pages", "parse", "corrupt"}
     d = tempfile.mkdtemp(prefix="cpu_warp_fuzz_")
     obj = os.path.join(d, "oracle.o")
     subprocess.check_call(["gcc", "-O2", "-c", "-o", obj, os.path.join(ROOT, "oracle", "snappy_oracle.c")])
     exe = {}
-    for name in ("window", "decode", "pages", "parse"):
+    for name, src in (("window", "run_window_kernel"), ("decode", "run_decode_kernel"), ("pages", "run_pages_kernel"),
+                      ("parse", "run_parse_kernel"), ("decode_parsed", "run_decode_parsed")):
         exe[name] = os.path.join(d, name)
         subprocess.check_call(["g++", "-O1", "-std=c++17", "-DSB200_CPU_EMU", "-DSB200_EXPERIMENTS", "-I" + os.path.join(ROOT, "tools", "cpu_warp"), "-o",
-                               exe[name], os.path.join(ROOT, "tools", "cpu_warp", "run_%s_kernel.cpp" % name), obj])
+                               exe[name], os.path.join(ROOT, "tools", "cpu_warp", "%s.cpp" % src), obj])
     raw, streams = [], []
     codec = pa.Codec("snappy")
     for i, b in enumerate(inputs(seed, count)):
@@ -86,26 +95,53 @@ def main():
             streams.append(q)
     bad = 0
 
-    def go(what, cmd, env=None):
+    def go(what, cmd, env=None, files=None):
+        """`files` (appended to cmd) are split over the CPU's cores"""
         nonlocal bad
-        p = subprocess.run(cmd, env=dict(os.environ, **(env or {})), capture_output=True, text=True)
-        wrong = [l for l in p.stdout.splitlines() if "0 mismatches" not in l and "no body" not in l and "header rejected" not in l]
-        print("%-44s %s" % (what, "ok" if p.returncode == 0 and not wrong else "MISMATCH"), flush=True)
-        for l in wrong[:5] + p.stderr.splitlines()[:5]:
+        groups = [files[k::os.cpu_count() or 1] for k in range(os.cpu_count() or 1)] if files else [[]]
+        with concurrent.futures.ThreadPoolExecutor(len(groups)) as ex:
+            runs = list(ex.map(lambda g: subprocess.run(cmd + g, env=dict(os.environ, **(env or {})), capture_output=True,
+                                                        text=True), [g for g in groups if g or not files]))
+        lines = [l for p in runs for l in p.stdout.splitlines()]
+        wrong = [l for l in lines if "0 mismatches" not in l and "no body" not in l and "header rejected" not in l]
+        failed = any(p.returncode != 0 for p in runs) or bool(wrong)
+        print("%-44s %s (%d lines)" % (what, "MISMATCH" if failed else "ok", len(lines)), flush=True)
+        for l in wrong[:5] + [l for p in runs for l in p.stderr.splitlines()][:5]:
             print("   ", l)
-        bad += p.returncode != 0 or bool(wrong)
+        bad += failed
 
-    for table, rules, ring in (("smem", 0, 1024), ("smem", 0, 2048), ("smem", 2, 4096), ("global", 0, 1024),
-                               ("global", 1, 2048), ("global", 2, 1024)):
-        go("window %s rules %d ring %d" % (table, rules, ring), [exe["window"]] + raw,
-           {"TABLE": table, "RULES": str(rules), "RING": str(ring)})
-    go("window + slowcont", [exe["window"]] + raw, {"SLOWCONT": "1"})
-    go("chain kernel", [exe["window"]] + raw, {"KERNEL": "chain"})
-    go("indexed decoder", [exe["decode"], "indexed"] + raw)
-    go("exact decoder on the streams", [exe["decode"], "exact"] + streams)
-    for rules in (0, 2):
-        go("pages rules %d" % rules, [exe["pages"]] + raw[3:40], {"RULES": str(rules)})
-    go("index-free parse", [exe["parse"]] + streams)
+    if "compress" in legs:
+        for table, rules, ring in (("smem", 0, 1024), ("smem", 0, 2048), ("smem", 2, 4096), ("global", 0, 1024),
+                                   ("global", 1, 2048), ("global", 2, 1024)):
+            go("window %s rules %d ring %d" % (table, rules, ring), [exe["window"]] + raw,
+               {"TABLE": table, "RULES": str(rules), "RING": str(ring)})
+        go("window + slowcont", [exe["window"]] + raw, {"SLOWCONT": "1"})
+        go("chain kernel", [exe["window"]] + raw, {"KERNEL": "chain"})
+    if "decode" in legs:
+        go("indexed decoder", [exe["decode"], "indexed"] + raw)
+        go("exact decoder on the streams", [exe["decode"], "exact"] + streams)
+    if "pages" in legs:
+        for rules in (0, 2):
+            go("pages rules %d" % rules, [exe["pages"]] + raw[3:40], {"RULES": str(rules)})
+    if "parse" in legs:
+        go("index-free parse", [exe["parse"]] + streams)
+    if "corrupt" in legs:
+        sys.path.insert(0, os.path.join(ROOT, "tests"))
+        from test_decode_corruption import mutations
+        rng = np.random.default_rng(seed)
+        mutated = []
+        for i, s in enumerate(streams):
+            data = open(s, "rb").read()
+            if i % 2 != (i // 2) % 2 or pyoracle.uncompressed_length(data) <= 65536:
+                continue  # multi-fragment streams only, Snappy.jl's and Google snappy's in turn
+            for k, (name, m) in enumerate(mutations(pyoracle, rng, os.path.basename(s), data, range(4))):
+                q = os.path.join(d, "m%05d_%s" % (len(mutated), name.replace("/", "__")))
+                open(q, "wb").write(m)
+                mutated.append(q)
+        go("corrupt streams, parsed decode", [exe["decode_parsed"], "parsed"], files=mutated)
+        for env in ({"PSHIFT": "9"}, {"PSHIFT": "12"}, {"CLEAN_CUTS": "0"}):
+            go("corrupt streams, parsed decode %s" % env, [exe["decode_parsed"], "parsed"], env, files=mutated[::3])
+        go("corrupt streams, pages", [exe["decode_parsed"], "pages"], files=mutated)
     print("inputs in", d)
     return 1 if bad else 0
 
