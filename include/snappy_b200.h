@@ -69,6 +69,14 @@ int snappy_b200_uncompressed_length(const uint8_t *in, size_t n, size_t *result)
  * ccall twin: snappy_uncompress (test/libsnappy.jl:25-28). */
 int snappy_b200_uncompress(const uint8_t *in, size_t n, uint8_t *out, size_t *out_len);
 
+/* snappy_validate_compressed_buffer / IsValidCompressedBuffer: would snappy_b200_uncompress accept `in`?  Returns
+ * exactly the status uncompress returns when the output capacity is unlimited: SNAPPY_B200_OK or one of the
+ * reference's statuses 2..6 (never BUFFER_TOO_SMALL); 8..10 for device problems only.  Takes no output buffer and
+ * writes nothing: the stream is judged on the GPU from its element headers and output positions (DESIGN.md section 4,
+ * "Validation").  `in` is a HOST pointer (pinned or pageable).
+ * ccall twin: snappy_validate_compressed_buffer (snappy-c). */
+int snappy_b200_validate_compressed_buffer(const uint8_t *in, size_t n);
+
 /* ---- device-resident API (the GB/s targets are quoted on these) --------------------------- */
 
 /* Same as snappy_b200_compress but d_in / d_out are DEVICE pointers; `stream` is a cudaStream_t
@@ -85,6 +93,14 @@ int snappy_b200_compress_device(const uint8_t *d_in, size_t n, uint8_t *d_out, s
  * back to the index-free path on any inconsistency.  Synchronises `stream`. */
 int snappy_b200_uncompress_device(const uint8_t *d_in, size_t n, uint8_t *d_out, size_t out_cap,
                                   size_t *out_len, const uint64_t *d_frag_index, void *stream);
+
+/* snappy_b200_validate_compressed_buffer on DEVICE memory.  d_frag_index (optional): a side index as for
+ * uncompress_device; right or wrong, it cannot change the result.  *uncompressed_len (optional) receives the claimed
+ * length when the header parses.  Device memory: the parse's O(n / parse chunk) plus 17 bytes per claimed 64 KiB
+ * fragment, never an output of `claimed` bytes.
+ * Synchronises `stream`. */
+int snappy_b200_validate_device(const uint8_t *d_in, size_t n, const uint64_t *d_frag_index,
+                                size_t *uncompressed_len, void *stream);
 
 /* ---- batched API: many independent streams (Parquet-page-like), one stream per page ------- */
 
@@ -105,6 +121,13 @@ int snappy_b200_uncompress_batched_device(const uint8_t *d_in, const uint64_t *d
                                           const uint32_t *d_in_sizes, size_t count, uint8_t *d_out,
                                           const uint64_t *d_out_offsets, const uint32_t *d_out_caps,
                                           uint32_t *d_out_sizes, int32_t *d_statuses, void *stream);
+
+/* Validation form of uncompress_batched_device: d_statuses[i] = what uncompress_batched_device reports for page i
+ * with unlimited room (never BUFFER_TOO_SMALL), d_claimed[i] = the page's claimed length (0 when its header does not
+ * parse).  No output.  DEVICE arrays of `count` entries.  Synchronises `stream`. */
+int snappy_b200_validate_batched_device(const uint8_t *d_in, const uint64_t *d_in_offsets,
+                                        const uint32_t *d_in_sizes, size_t count, uint32_t *d_claimed,
+                                        int32_t *d_statuses, void *stream);
 
 /* ---- shard API: multi-GPU sharding on whole-fragment boundaries --------------------------- */
 

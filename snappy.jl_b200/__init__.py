@@ -9,7 +9,7 @@ fails with SnappyError when no sm_100 GPU is usable.
 """
 from . import _abi
 from .api import (SnappyError, pack_index, unpack_index, set_rules, compress, compress_np, encode32, find_match_length,
-                  length_uncompressed, maxlength_compressed, parse32, uncompress, uncompress_np)
+                  length_uncompressed, maxlength_compressed, parse32, uncompress, uncompress_np, validate)
 
 K_BLOCK_SIZE = 65536          # src/internal.jl:31
 K_INPUT_MARGIN_BYTES = 15     # src/internal.jl:32

@@ -38,6 +38,9 @@ SIGNATURES = {
     "snappy_b200_compress": (ctypes.c_int, [_vp, _sz, _vp, _szp]),
     "snappy_b200_uncompressed_length": (ctypes.c_int, [_vp, _sz, _szp]),
     "snappy_b200_uncompress": (ctypes.c_int, [_vp, _sz, _vp, _szp]),
+    "snappy_b200_validate_compressed_buffer": (ctypes.c_int, [_vp, _sz]),
+    "snappy_b200_validate_device": (ctypes.c_int, [_vp, _sz, _vp, _szp, _vp]),
+    "snappy_b200_validate_batched_device": (ctypes.c_int, [_vp, _vp, _vp, _sz, _vp, _vp, _vp]),
     "snappy_b200_compress_device": (ctypes.c_int, [_vp, _sz, _vp, _sz, _szp, _vp, _vp]),
     "snappy_b200_uncompress_device": (ctypes.c_int, [_vp, _sz, _vp, _sz, _szp, _vp, _vp]),
     "snappy_b200_compress_batched_device": (ctypes.c_int, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp]),

@@ -86,6 +86,17 @@ def uncompress(data):
     return uncompress_np(data).tobytes()
 
 
+def validate(data):
+    """snappy_validate_compressed_buffer / IsValidCompressedBuffer: the status `uncompress(data)` would end with --
+    0 when it would succeed, else the reference's status 2..6 (`SnappyError(status)` carries its message).  Nothing is
+    decoded and no output is allocated; raises SnappyError only for CUDA / device problems."""
+    a = _as_u8(data)
+    rc = _abi.lib().snappy_b200_validate_compressed_buffer(_ptr(a), a.size)
+    if rc >= _abi.BUFFER_TOO_SMALL:
+        raise SnappyError(rc, _abi.last_error())
+    return rc
+
+
 def parse32(buf, offset=0):
     """varint.jl:12-37 with a 0-based offset: returns (value, index past the varint)."""
     a = _as_u8(buf)

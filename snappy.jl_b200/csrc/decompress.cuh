@@ -107,6 +107,9 @@ __device__ __forceinline__ void warp_copy_backref(u8* out, u64 op, u32 offset, u
 // Range form: elements from *ip up to (not including) ip_stop, output position *op; returns the status of the first
 // failing element (ST_OK if none).  The whole-stream decoder is the range [ip0, L) from op = 0 plus the final length
 // check (src/Snappy.jl:50).
+// kWrite = false: validation only -- the same walk, the same checks and the same op, but no byte is written and `out`
+// is never touched (it may be null).
+template <bool kWrite = true>
 __device__ __forceinline__ int decode_exact_range(const u8* __restrict__ in, u64 L, u64& ip, u64 ip_stop,
                                                   u8* __restrict__ out, u64 n, u64& op, u32 lane) {
     while (ip < ip_stop && ip + 1 < L) {  // src/internal.jl:416
@@ -118,26 +121,27 @@ __device__ __forceinline__ int decode_exact_range(const u8* __restrict__ in, u64
         if (e.is_copy) {
             if (e.offset == 0 || (u64)e.offset > op) return ST_CORRUPT_COPY_OFFSET;  // :499
             if (n - op < e.len) return ST_CORRUPT_COPY_LENGTH;                       // :505
-            warp_copy_backref(out, op, e.offset, e.len, lane);
+            if (kWrite) warp_copy_backref(out, op, e.offset, e.len, lane);
             op += e.len;
         } else {
             // avail_in may be negative when the header bytes ran past the end (:517-518)
             long long avail_in = (long long)L - (long long)ip;
             if (n - op < (u64)e.len || avail_in < (long long)e.len) return ST_CORRUPT_LITERAL;
-            warp_copy_literal(out + op, in + ip, e.len, lane);
+            if (kWrite) warp_copy_literal(out + op, in + ip, e.len, lane);
             op += e.len;
             ip += e.len;
         }
-        __syncwarp();
+        if (kWrite) __syncwarp();
     }
     return ST_OK;
 }
 
+template <bool kWrite = true>
 __device__ __forceinline__ int decode_exact_warp(const u8* __restrict__ in, u64 L, u64 ip0,
                                                  u8* __restrict__ out, u64 n, u32 lane,
                                                  u64& produced) {
     u64 ip = ip0, op = 0;
-    int status = decode_exact_range(in, L, ip, L, out, n, op, lane);
+    int status = decode_exact_range<kWrite>(in, L, ip, L, out, n, op, lane);
     if (status == ST_OK && op != n) status = ST_INVALID_INPUT;  // src/Snappy.jl:50
     produced = op;
     return status;
@@ -149,6 +153,19 @@ k_decode_serial(const u8* __restrict__ in, u64 L, u64 ip0, u8* __restrict__ out,
     const u32 lane = lane_id();
     u64 produced;
     int status = decode_exact_warp(in, L, ip0, out, n, lane, produced);
+    if (lane == 0) {
+        res->status = status;
+        res->produced = produced;
+        res->err_op = produced;
+    }
+}
+
+// Status-only twin of k_decode_serial (snappy_b200_validate_*): no output buffer.
+__global__ void __launch_bounds__(32)
+k_validate_serial(const u8* __restrict__ in, u64 L, u64 ip0, u64 n, DecodeResult* __restrict__ res) {
+    const u32 lane = lane_id();
+    u64 produced;
+    int status = decode_exact_warp<false>(in, L, ip0, nullptr, n, lane, produced);
     if (lane == 0) {
         res->status = status;
         res->produced = produced;
@@ -201,6 +218,8 @@ __device__ __forceinline__ void decode_tag_fast(u32 c, u32 tag4, u32& len, u32& 
     offset = (kind == 1) ? (((c >> 5) << 8) | v) : v;
 }
 
+// kWrite = false: the window parse, chain, scan and every check, without the execute loop (validation; `o` unused).
+template <bool kWrite = true>
 __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 ip, const u64 ie,
                                                  u8* __restrict__ o, const u32 on, const u32 lane) {
     if (ie - ip > 0xfffffff0ull) return false;
@@ -275,6 +294,11 @@ __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 
         const u32 exitm = __ballot_sync(kFullMask, mine && leaves);
         if (__any_sync(kFullMask, bad) || exitm == 0 || total > on - op) return false;
         const u32 nbase = __shfl_sync(kFullMask, p + size, (u32)__ffs((int)exitm) - 1u);
+        if (!kWrite) {
+            op += total;
+            base = nbase;
+            continue;
+        }
         // ---- execute
         const u32 lsrc = p + hdr;  // literal bytes start behind the header
         // highest output byte (exclusive) the element reads; literals read none
@@ -398,16 +422,39 @@ k_decode_fragments(const u8* __restrict__ in, const u64* __restrict__ frag_off, 
     }
 }
 
+// Validation over a side index: one warp per 64 KiB fragment with the per-fragment rules of k_decode_fragments
+// (fragment 0 starts behind the header, the last ends at in_end, fragment f is exactly in[frag_off[f] ..
+// frag_off[f+1]) with exactly its output length, no copy reaches before the fragment), but no output: a fragment that
+// is not clean raises res->fallback and the index-free chain decides.
+__global__ void __launch_bounds__(kDecodeWarpsPerCta * 32)
+k_validate_fragments(const u8* __restrict__ in, const u64* __restrict__ frag_off, u32 nfrag, u64 in_begin,
+                     u64 in_end, u64 out_len, DecodeResult* __restrict__ res) {
+    const u32 lane = lane_id();
+    const u32 f = blockIdx.x * kDecodeWarpsPerCta + (threadIdx.x >> 5);
+    if (f >= nfrag) return;
+    const u64 ip = frag_off[f];
+    const u64 ie = frag_off[f + 1];
+    const u64 ob = (u64)f * kBlockSize;
+    u64 oe = ob + kBlockSize;
+    if (oe > out_len) oe = out_len;
+    const u32 on = oe >= ob ? (u32)(oe - ob) : 0u;
+    bool ok = (ie >= ip) && (ie <= in_end) && (f != 0 || ip == in_begin) && (f != nfrag - 1 || ie == in_end) &&
+              (oe >= ob);
+    if (ok) ok = decode_fast_warp<false>(in, ip, ie, nullptr, on, lane);
+    if (!ok && lane == 0) atomicOr(&res->fallback, 1u);
+}
+
 // Status arbiter, bounded: only the tiles the parallel decoder rejected (tile_flags) are decoded again, one warp,
 // element by element with the reference's checks (decode_exact_range), in stream order.  Every tile before the first
 // rejected one passed the (stricter) clean-tile validation, so its bytes are final and the reference accepts it too:
 // the first error this walk meets is the reference's first error.  A rejected tile that decodes fine in whole-stream
 // terms (a copy that reaches into an earlier tile) is simply complete afterwards.  The walk goes on through the
 // following tiles until it stands exactly on the start of a tile that was not rejected.
-__global__ void __launch_bounds__(32)
-k_decode_serial_tiles(const u8* __restrict__ in, u64 L, const u64* __restrict__ index,
-                      const u64* __restrict__ out_start, u32 nfrag, const u8* __restrict__ tile_flags,
-                      u8* __restrict__ out, u64 n, DecodeResult* __restrict__ res) {
+template <bool kWrite>
+__device__ __forceinline__ void serial_tiles_walk(const u8* __restrict__ in, u64 L, const u64* __restrict__ index,
+                                                  const u64* __restrict__ out_start, u32 nfrag,
+                                                  const u8* __restrict__ tile_flags, u8* __restrict__ out, u64 n,
+                                                  DecodeResult* __restrict__ res) {
     const u32 lane = lane_id();
     int status = ST_OK;
     u64 ip = 0, op = 0;
@@ -427,7 +474,7 @@ k_decode_serial_tiles(const u8* __restrict__ in, u64 L, const u64* __restrict__ 
         for (;;) {
             // one element at a time, so that the walk can stop on a tile start
             u64 stop = ip + 1;
-            status = decode_exact_range(in, L, ip, stop, out, n, op, lane);
+            status = decode_exact_range<kWrite>(in, L, ip, stop, out, n, op, lane);
             if (status != ST_OK) break;
             if (ip + 1 >= L) {  // end of the stream (a lone trailing byte is ignored, src/internal.jl:416)
                 ran_to_end = true;
@@ -446,6 +493,21 @@ k_decode_serial_tiles(const u8* __restrict__ in, u64 L, const u64* __restrict__ 
         res->produced = op;
         res->err_op = op;
     }
+}
+
+__global__ void __launch_bounds__(32)
+k_decode_serial_tiles(const u8* __restrict__ in, u64 L, const u64* __restrict__ index,
+                      const u64* __restrict__ out_start, u32 nfrag, const u8* __restrict__ tile_flags,
+                      u8* __restrict__ out, u64 n, DecodeResult* __restrict__ res) {
+    serial_tiles_walk<true>(in, L, index, out_start, nfrag, tile_flags, out, n, res);
+}
+
+// Status-only twin (validation): the same walk from the same starts with the same checks, tracking op only.
+__global__ void __launch_bounds__(32)
+k_validate_serial_tiles(const u8* __restrict__ in, u64 L, const u64* __restrict__ index,
+                        const u64* __restrict__ out_start, u32 nfrag, const u8* __restrict__ tile_flags, u64 n,
+                        DecodeResult* __restrict__ res) {
+    serial_tiles_walk<false>(in, L, index, out_start, nfrag, tile_flags, nullptr, n, res);
 }
 
 // Batched pages: one warp per independent stream (own varint header).  Fast path first; the exact
@@ -490,6 +552,32 @@ k_decode_pages(const u8* __restrict__ in, const u64* __restrict__ in_off,
     if (lane == 0) {
         statuses[pg] = status;
         out_size[pg] = (status == ST_OK) ? claimed : 0;
+    }
+}
+
+// Status-only twin of k_decode_pages (snappy_b200_validate_batched_device): no output, no capacity; writes the claimed
+// length (0 when the header does not parse) and the reference's status of every page.
+__global__ void __launch_bounds__(kDecodeWarpsPerCta * 32)
+k_validate_pages(const u8* __restrict__ in, const u64* __restrict__ in_off, const u32* __restrict__ in_size, u32 count,
+                 u32* __restrict__ claimed_out, int* __restrict__ statuses) {
+    const u32 lane = lane_id();
+    const u32 pg = blockIdx.x * kDecodeWarpsPerCta + (threadIdx.x >> 5);
+    if (pg >= count) return;
+    const u8* pin = in + in_off[pg];
+    const u64 L = in_size[pg];
+    u32 claimed = 0, hdr = 0;
+    int status = parse_varint_dev(pin, L, claimed, hdr);
+    if (status == ST_OK) {
+        bool ok = (claimed <= kBlockSize) && decode_fast_warp<false>(pin, hdr, L, nullptr, claimed, lane);
+        if (!ok) {
+            u64 produced;
+            __syncwarp();
+            status = decode_exact_warp<false>(pin, L, hdr, nullptr, claimed, lane, produced);
+        }
+    }
+    if (lane == 0) {
+        statuses[pg] = status;
+        claimed_out[pg] = status == ST_BAD_VARINT ? 0u : claimed;
     }
 }
 

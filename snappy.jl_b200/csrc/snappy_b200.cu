@@ -1155,6 +1155,121 @@ int uncompress_device_locked(Context& c, const u8* d_in, size_t n, u8* d_out, si
     return decode_exact_locked(c, d_in, n, hdr, d_out, claimed, st);
 }
 
+// ---- validation (snappy_b200_validate_*): uncompress_device_locked's chain, status only --------------------------
+// The same paths in the same order with the same verdicts, but no output buffer: the device memory is the parse's
+// (O(n / parse chunk)) plus the tile index (O(claimed / 64 KiB)), never O(claimed).
+
+// status-only whole-stream walk (path 3)
+int validate_exact_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, cudaStream_t st) {
+    DecodeResult* res = (DecodeResult*)c.result.p;
+    k_validate_serial<<<1, 32, 0, st>>>(d_in, (u64)n, (u64)hdr, (u64)claimed, res);
+    c.last_launches[1] += 1;
+    CU(cudaGetLastError());
+    DecodeResult* h = (DecodeResult*)((u8*)c.pinned + 128);
+    CU(cudaMemcpyAsync(h, res, sizeof(DecodeResult), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return h->status;
+}
+
+// path 0: every fragment of the side index is clean -> OK; -1 when some fragment is not (caller: the parse)
+int validate_indexed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, const u64* d_index,
+                            cudaStream_t st) {
+    const u32 nfrag = frag_count(claimed);
+    if (nfrag == 0) return -1;
+    CU(cudaMemsetAsync(c.result.p, 0, sizeof(DecodeResult), st));
+    if (c.opt.timing) CU(cudaEventRecord(c.ev[2], st));
+    const u32 grid = (nfrag + kDecodeWarpsPerCta - 1) / kDecodeWarpsPerCta;
+    k_validate_fragments<<<grid, kDecodeWarpsPerCta * 32, 0, st>>>(d_in, d_index, nfrag, (u64)hdr, (u64)n,
+                                                                    (u64)claimed, (DecodeResult*)c.result.p);
+    c.last_launches[1] += 1;
+    return decode_finish(c, st, false);
+}
+
+// decode_parsed_locked without the decode.  The parse's first failing element and its length check decide every
+// stream whose chain it followed to the end (path 1): a complete, error-free parse whose lengths add up means the
+// reference accepts the stream, because its three element checks depend on the element header and the output position
+// only (k_build_index).  A parse that lost the chain hands over to the status-only walk from the last tile start it
+// reached (path 2).  -1: nothing usable came out of the parse (caller: whole-stream walk).
+int validate_parsed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, cudaStream_t st) {
+    const u32 nfrag = frag_count(claimed);
+    if (nfrag == 0 || n <= hdr) return -1;
+    CU(c.index.ensure(((size_t)nfrag + 1) * 8));
+    CU(c.index_out.ensure(((size_t)nfrag + 1) * 8));
+    CU(c.tile_flags.ensure((size_t)nfrag + 64));
+    u64* idx = (u64*)c.index.p;
+    u64* ost = (u64*)c.index_out.p;
+    u8* tf = (u8*)c.tile_flags.p;
+    CU(cudaMemsetAsync(idx, 0xff, ((size_t)nfrag + 1) * 8, st));
+    CU(cudaMemsetAsync(ost, 0xff, ((size_t)nfrag + 1) * 8, st));
+    u64* hseed = (u64*)((u8*)c.pinned + 3072);  // tile 0 starts behind the header whatever the parse finds
+    hseed[0] = hdr;
+    hseed[1] = 0;
+    hseed[2] = claimed;
+    CU(cudaMemcpyAsync(idx, hseed, 8, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(ost, hseed + 1, 8, cudaMemcpyHostToDevice, st));
+    u64 ex = 0, total = 0, pflags = 0, first_err = ~0ull;
+    int rc = build_index_segment(c, d_in, n, hdr, n, 0, nfrag, st, &ex, &total, ost, &pflags, (u64)claimed, &first_err);
+    if (rc != 0) return rc;
+    c.last_path = 1;
+    if (first_err != ~0ull) return (int)(first_err & 7);
+    if (!(pflags & (PF_ANOMALY | PF_BROKEN)))
+        return total == claimed ? SNAPPY_B200_OK : SNAPPY_B200_INVALID_INPUT;  // src/Snappy.jl:50
+    // the chain broke: tiles [0, tvalid) have both ends in the index; the walk starts at the last entry the parse wrote
+    // and runs to the end of the stream (the length check) or to the first failing element
+    CU(cudaMemcpyAsync(ost + nfrag, hseed + 2, 8, cudaMemcpyHostToDevice, st));
+    u32* d_first = (u32*)((u8*)c.result.p + 128);
+    u32* h_first = (u32*)((u8*)c.pinned + 3104);
+    *h_first = nfrag + 1;
+    CU(cudaMemcpyAsync(d_first, h_first, 4, cudaMemcpyHostToDevice, st));
+    k_first_missing<<<(nfrag + 1 + 255) / 256, 256, 0, st>>>(idx, nfrag, (u64)n, d_first);
+    CU(cudaMemcpyAsync(h_first, d_first, 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const u32 first = *h_first;
+    u32 tvalid = first == 0 ? 0u : (first > nfrag ? nfrag : first - 1);
+    if (first <= nfrag && first > 0 && tvalid > 0) tvalid = first - 1;
+    c.last_path = 2;
+    CU(cudaMemsetAsync(tf, 0, (size_t)nfrag + 64, st));
+    if (tvalid < nfrag) CU(cudaMemsetAsync(tf + tvalid, 1, nfrag - tvalid, st));
+    CU(cudaMemsetAsync(tf + nfrag - 1, 1, 1, st));  // the walk must see the end of the stream (length check)
+    CU(cudaMemsetAsync(c.result.p, 0, sizeof(DecodeResult), st));
+    DecodeResult* res = (DecodeResult*)c.result.p;
+    k_validate_serial_tiles<<<1, 32, 0, st>>>(d_in, (u64)n, idx, ost, nfrag, tf, (u64)claimed, res);
+    c.last_launches[1] += 2;
+    CU(cudaGetLastError());
+    DecodeResult* h = (DecodeResult*)((u8*)c.pinned + 128);
+    CU(cudaMemcpyAsync(h, res, sizeof(DecodeResult), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return h->status;
+}
+
+// uncompress_device_locked, step for step, without an output: the status uncompress returns when out_cap is unlimited
+int validate_device_locked(Context& c, const u8* d_in, size_t n, const u64* d_index, size_t* claimed_out,
+                           cudaStream_t st) {
+    c.last_launches[1] = 0;
+    u8* hb = (u8*)c.pinned + 256;
+    const size_t hn = n < 5 ? n : 5;
+    if (hn) {
+        CU(cudaMemcpyAsync(hb, d_in, hn, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    u32 claimed = 0;
+    size_t hdr = 0;
+    int rc = parse_varint(hb, hn, &claimed, &hdr);
+    if (rc != SNAPPY_B200_OK) return rc;
+    if (claimed_out) *claimed_out = claimed;
+    if (c.opt.decode_variant != 1) {
+        if (d_index) {  // as in uncompress: a wrong index only costs the fragment pass
+            c.last_path = 0;
+            rc = validate_indexed_locked(c, d_in, n, hdr, claimed, d_index, st);
+            if (rc >= 0) return rc;
+        }
+        rc = validate_parsed_locked(c, d_in, n, hdr, claimed, st);
+        if (rc >= 0) return rc;
+    }
+    c.last_path = 3;
+    return validate_exact_locked(c, d_in, n, hdr, claimed, st);
+}
+
 // Takes a lane of the addressed device for the duration of a call: resolves the device, makes it current (the
 // caller's current device is restored on exit), picks a free lane or creates one.
 struct Locked {
@@ -1333,6 +1448,14 @@ int snappy_b200_uncompress_device(const uint8_t* d_in, size_t n, uint8_t* d_out,
     if (L.rc != SNAPPY_B200_OK) return L.rc;
     return uncompress_device_locked(*L.c, d_in, n, d_out, out_cap, out_len, (const u64*)d_frag_index,
                                     (cudaStream_t)stream);
+}
+
+int snappy_b200_validate_device(const uint8_t* d_in, size_t n, const uint64_t* d_frag_index, size_t* uncompressed_len,
+                                void* stream) {
+    if (!d_in && n) return SNAPPY_B200_BAD_ARGUMENT;
+    Locked L;
+    if (L.rc != SNAPPY_B200_OK) return L.rc;
+    return validate_device_locked(*L.c, d_in, n, (const u64*)d_frag_index, uncompressed_len, (cudaStream_t)stream);
 }
 
 extern "C++" {
@@ -2027,6 +2150,36 @@ int snappy_b200_uncompress(const uint8_t* in, size_t n, uint8_t* out, size_t* ou
     return SNAPPY_B200_OK;
 }
 
+// Host-buffer validation: the stream goes up as the host uncompress sends it (pinned: one copy; pageable: through the
+// bounce slots), then the device chain judges it.  No output buffer on either side.
+int snappy_b200_validate_compressed_buffer(const uint8_t* in, size_t n) {
+    if (!in && n) return SNAPPY_B200_BAD_ARGUMENT;
+    u32 claimed = 0;
+    size_t hdr = 0;
+    int rc = parse_varint(in, n, &claimed, &hdr);  // src/Snappy.jl:47
+    if (rc != SNAPPY_B200_OK) return rc;
+    Locked L;
+    if (L.rc != SNAPPY_B200_OK) return L.rc;
+    Context& c = *L.c;
+    CU(c.stage_in.ensure(n + 16));
+    const bool pg_in = c.opt.pin_host && is_pageable(in);
+    if (pg_in) {
+        int rb = bounce_init(c);
+        if (rb != SNAPPY_B200_OK) return rb;
+    }
+    {
+        PipeGuard guard{c};
+        Uploader up(c, pg_in, n, 0);
+        int ru = up.put((u8*)c.stage_in.p, in, n);
+        if (ru == SNAPPY_B200_OK) ru = up.sync();
+        if (ru != SNAPPY_B200_OK) return ru;
+        CU(cudaStreamSynchronize(c.s_h2d));
+        guard.drained = true;
+    }
+    size_t claimed_len = 0;
+    return validate_device_locked(c, (const u8*)c.stage_in.p, n, nullptr, &claimed_len, c.s_comp);
+}
+
 int snappy_b200_compress_shard_device(const uint8_t* d_shard, size_t shard_len, uint64_t total_len,
                                       uint8_t* d_out, size_t out_cap, size_t* out_len,
                                       uint32_t* d_frag_sizes, void* stream) {
@@ -2289,6 +2442,30 @@ int snappy_b200_uncompress_batched_device(const uint8_t* d_in, const uint64_t* d
     k_decode_pages<<<grid, kDecodeWarpsPerCta * 32, 0, st>>>(d_in, d_in_offsets, d_in_sizes, (u32)count,
                                                              d_out, d_out_offsets, d_out_caps,
                                                              d_out_sizes, d_statuses);
+    if (c.opt.timing) {
+        CU(cudaEventRecord(c.ev[3], st));
+        c.ev_pending[1] = true;
+    }
+    c.last_launches[1] = 1;
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(st));
+    harvest_timing(c, 1);
+    return SNAPPY_B200_OK;
+}
+
+int snappy_b200_validate_batched_device(const uint8_t* d_in, const uint64_t* d_in_offsets, const uint32_t* d_in_sizes,
+                                        size_t count, uint32_t* d_claimed, int32_t* d_statuses, void* stream) {
+    if (count == 0) return SNAPPY_B200_OK;
+    if (!d_in || !d_in_offsets || !d_in_sizes || !d_claimed || !d_statuses) return SNAPPY_B200_BAD_ARGUMENT;
+    if (count > 0x7fffffffull) return SNAPPY_B200_BAD_ARGUMENT;
+    Locked L;
+    if (L.rc != SNAPPY_B200_OK) return L.rc;
+    Context& c = *L.c;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (c.opt.timing) CU(cudaEventRecord(c.ev[2], st));
+    const unsigned grid = (unsigned)((count + kDecodeWarpsPerCta - 1) / kDecodeWarpsPerCta);
+    k_validate_pages<<<grid, kDecodeWarpsPerCta * 32, 0, st>>>(d_in, d_in_offsets, d_in_sizes, (u32)count, d_claimed,
+                                                               d_statuses);
     if (c.opt.timing) {
         CU(cudaEventRecord(c.ev[3], st));
         c.ev_pending[1] = true;

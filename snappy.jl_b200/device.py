@@ -72,6 +72,20 @@ def uncompress_device(stream, out=None, index=None, claimed=None):
     return out[: out_len.value]
 
 
+def validate_device(stream, index=None):
+    """Would uncompress_device(stream, index=index) succeed?  Returns (status, claimed): status 0 or the reference's
+    2..6, exactly what uncompress_device reports with unlimited room; claimed is the header's length, None when the
+    header does not parse.  No output is allocated; `index` (optional side index) cannot change the result."""
+    claimed = ctypes.c_size_t(0)
+    with torch.cuda.device(stream.device):
+        _abi.lib().snappy_b200_init(stream.device.index)
+        rc = _abi.lib().snappy_b200_validate_device(_dev_ptr(stream), stream.numel(), _dev_ptr(index),
+                                                    ctypes.byref(claimed), _stream_ptr(stream.device))
+    if rc >= _abi.BUFFER_TOO_SMALL:
+        raise SnappyError(rc, _abi.last_error())
+    return rc, (None if rc == _abi.BAD_VARINT else claimed.value)
+
+
 def compress_shard_device(shard, total_len, out=None, want_sizes=False):
     """Compress a run of whole fragments of a stream whose total length is `total_len`
     (elements only, no varint header).  Returns (bytes_view, frag_sizes or None)."""
@@ -180,6 +194,22 @@ def uncompress_batched_device(data, in_offsets, in_sizes, out, out_offsets, out_
             _dev_ptr(out_offsets), _dev_ptr(out_caps), _dev_ptr(out_sizes), _dev_ptr(statuses),
             _stream_ptr(dev)))
     return out_sizes, statuses
+
+
+def validate_batched_device(data, in_offsets, in_sizes):
+    """Validation form of uncompress_batched_device (no output).  Returns (statuses, claimed) int32 device tensors:
+    per page what uncompress_batched_device reports with unlimited room, and the header's length (0 when it does not
+    parse)."""
+    count = in_sizes.numel()
+    dev = data.device
+    claimed = torch.zeros(count, dtype=torch.int32, device=dev)
+    statuses = torch.zeros(count, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _abi.lib().snappy_b200_init(dev.index)
+        _check(_abi.lib().snappy_b200_validate_batched_device(
+            _dev_ptr(data), _dev_ptr(in_offsets), _dev_ptr(in_sizes), count, _dev_ptr(claimed), _dev_ptr(statuses),
+            _stream_ptr(dev)))
+    return statuses, claimed
 
 
 def last_kernel_ms(which):

@@ -82,6 +82,20 @@ function uncompress(input::Vector{UInt8})
     return output
 end
 
+"""
+    validate(input::Vector{UInt8}) -> Int
+
+The status `uncompress(input)` would end with, without decoding: 0 when it would succeed, else the reference's
+status 2..6 (`snappy_b200_status_string` gives its message).  No output buffer.  Device problems raise.
+"""
+function validate(input::Vector{UInt8})
+    status = GC.@preserve input begin
+        ccall((:snappy_b200_validate_compressed_buffer, LIB), Cint, (Ptr{UInt8}, Csize_t), input, length(input))
+    end
+    status >= 7 && _check(status)
+    return Int(status)
+end
+
 # test/runtests.jl:172 calls Snappy.find_match_length(c, i1, i2, limit) with 1-based indices and an
 # inclusive limit; the C helper is 0-based with an exclusive limit.
 function find_match_length(a::Vector{UInt8}, i1::Integer, i2::Integer, limit::Integer)

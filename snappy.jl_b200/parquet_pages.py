@@ -205,6 +205,35 @@ def uncompress_pages(file_bytes, pages=None):
     return pages, out.cpu().numpy(), offs
 
 
+def validate_pages(file_bytes, pages=None):
+    """Would uncompress_pages accept each page?  ONE batched validation call on the GPU (no output is allocated or
+    written).  Returns (pages, statuses): statuses[i] is 0 or the reference's status 2..6 of page i's Snappy stream,
+    INVALID_INPUT (2) as well when the stream's length disagrees with the page header's uncompressed size, and -1 for
+    pages uncompress_pages does not decode (another codec, or no compressed bytes)."""
+    import torch
+    from . import _abi, device
+    if pages is None:
+        pages = list_pages(file_bytes)
+    sel = [i for i, p in enumerate(pages) if pages[i]["codec"] == SNAPPY and pages[i]["compressed"] > 0]
+    for i in sel:
+        p = pages[i]
+        if not (0 <= p["stream"] and p["stream"] + p["compressed"] <= len(file_bytes) and p["compressed"] < 1 << 31):
+            raise ValueError("page stream [%d, +%d) does not fit the file image (%d bytes)"
+                             % (p["stream"], p["compressed"], len(file_bytes)))
+    statuses = np.full(len(pages), -1, dtype=np.int32)
+    if not sel:
+        return pages, statuses
+    d_file = torch.from_numpy(np.frombuffer(bytes(file_bytes), dtype=np.uint8).copy()).cuda()
+    in_off = torch.tensor([pages[i]["stream"] for i in sel], dtype=torch.int64, device="cuda")
+    in_sz = torch.tensor([pages[i]["compressed"] for i in sel], dtype=torch.int32, device="cuda")
+    st, claimed = device.validate_batched_device(d_file, in_off, in_sz)
+    st, claimed = st.cpu().numpy(), claimed.cpu().numpy().astype(np.uint32)
+    for k, i in enumerate(sel):
+        ok_len = int(claimed[k]) == pages[i]["uncompressed"]
+        statuses[i] = _abi.INVALID_INPUT if st[k] == _abi.OK and not ok_len else st[k]
+    return pages, statuses
+
+
 def compress_pages(page_bytes):
     """Writer side: a list of uncompressed page bodies -> list of SNAPPY page bodies (bytes), one
     independent stream per page, all pages in ONE batched GPU call."""
