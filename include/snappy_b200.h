@@ -102,6 +102,33 @@ int snappy_b200_uncompress_device(const uint8_t *d_in, size_t n, uint8_t *d_out,
 int snappy_b200_validate_device(const uint8_t *d_in, size_t n, const uint64_t *d_frag_index,
                                 size_t *uncompressed_len, void *stream);
 
+/* Bytes [offset, offset + length) of what snappy_b200_uncompress_device would write, into d_out (length bytes of
+ * room; nothing outside [d_out, d_out + length) is written).  offset + length > claimed length -> BAD_ARGUMENT.
+ * Errors are checked in this order: the header (BAD_VARINT), the range (BAD_ARGUMENT), the stream.
+ * Without an index (d_frag_index NULL) the call is exact: it returns what snappy_b200_uncompress_device returns with
+ * unlimited room, for every input and every length (0 included), and on OK the bytes of that call's output.  It reads
+ * every element header of the stream but decodes only the tiles that overlap the range.
+ * With an index the call TRUSTS it for where the touched fragments offset / 65536 .. (offset + length - 1) / 65536
+ * start: each of them gets every per-fragment check of the indexed decoder over its whole length (starts at its entry,
+ * ends exactly at the next one, produces exactly its 64 KiB or the tail, no copy reaches before it), and if all pass
+ * the call returns OK without looking at the other fragments -- so a stream corrupt only outside the range still reads
+ * fine, and an empty range touches no fragment.  If any touched fragment fails, the call proceeds as the no-index
+ * call.  To have the whole stream judged, pass no index or call snappy_b200_validate_device.
+ * Device memory: the parse's arrays and one tile of scratch; an output of the claimed length only for a stream shown to
+ * be valid whose range could not be decoded from its tiles.  Synchronises `stream`. */
+int snappy_b200_uncompress_range_device(const uint8_t *d_in, size_t n, const uint64_t *d_frag_index,
+                                        uint64_t offset, size_t length, uint8_t *d_out, void *stream);
+
+/* `count` independent range reads (several may name the same stream) in one pass.  HOST arrays of `count` entries
+ * whose pointer members are DEVICE pointers (d_frag_indexes itself, or entries of it, may be NULL); statuses
+ * (HOST) receives what snappy_b200_uncompress_range_device returns for each request.  Returns OK when the batch
+ * ran, BAD_ARGUMENT when the indexed requests touch more than 2^31 - 1 fragments in all.  One launch decodes the touched fragments of every request that has an index; the others, and those with a
+ * rejected fragment, go through the single-range chain without the index.  Synchronises `stream`. */
+int snappy_b200_uncompress_ranges_device(const uint8_t *const *d_ins, const size_t *in_lens,
+                                         const uint64_t *const *d_frag_indexes, const uint64_t *offsets,
+                                         const size_t *lengths, uint8_t *const *d_outs, size_t count,
+                                         int *statuses, void *stream);
+
 /* ---- batched API: many independent streams (Parquet-page-like), one stream per page ------- */
 
 /* Page i is d_in + in_offsets[i], in_sizes[i] bytes; its stream (own varint header, own table

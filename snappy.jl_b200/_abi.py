@@ -41,6 +41,8 @@ SIGNATURES = {
     "snappy_b200_validate_compressed_buffer": (ctypes.c_int, [_vp, _sz]),
     "snappy_b200_validate_device": (ctypes.c_int, [_vp, _sz, _vp, _szp, _vp]),
     "snappy_b200_validate_batched_device": (ctypes.c_int, [_vp, _vp, _vp, _sz, _vp, _vp, _vp]),
+    "snappy_b200_uncompress_range_device": (ctypes.c_int, [_vp, _sz, _vp, ctypes.c_uint64, _sz, _vp, _vp]),
+    "snappy_b200_uncompress_ranges_device": (ctypes.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp, _vp]),
     "snappy_b200_compress_device": (ctypes.c_int, [_vp, _sz, _vp, _sz, _szp, _vp, _vp]),
     "snappy_b200_uncompress_device": (ctypes.c_int, [_vp, _sz, _vp, _sz, _szp, _vp, _vp]),
     "snappy_b200_compress_batched_device": (ctypes.c_int, [_vp, _vp, _vp, _sz, _vp, _vp, _vp, _vp]),

@@ -219,9 +219,13 @@ __device__ __forceinline__ void decode_tag_fast(u32 c, u32 tag4, u32& len, u32& 
 }
 
 // kWrite = false: the window parse, chain, scan and every check, without the execute loop (validation; `o` unused).
-template <bool kWrite = true>
+// kClip (range decoding): only o[0 .. lim) is written.  Elements wholly below lim run as usual, the one that crosses lim
+// is cut to lim - dst bytes, and every later element is parsed and checked but not executed.  A copy reads only bytes
+// below its own destination, so the bytes below lim never depend on the elements that are cut or skipped.
+template <bool kWrite = true, bool kClip = false>
 __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 ip, const u64 ie,
-                                                 u8* __restrict__ o, const u32 on, const u32 lane) {
+                                                 u8* __restrict__ o, const u32 on, const u32 lane,
+                                                 const u32 lim = 0xffffffffu) {
     if (ie - ip > 0xfffffff0ull) return false;
     const u8* __restrict__ src = in + ip;   // all positions below are relative to the run start
     const u32 nin = (u32)(ie - ip);
@@ -294,20 +298,21 @@ __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 
         const u32 exitm = __ballot_sync(kFullMask, mine && leaves);
         if (__any_sync(kFullMask, bad) || exitm == 0 || total > on - op) return false;
         const u32 nbase = __shfl_sync(kFullMask, p + size, (u32)__ffs((int)exitm) - 1u);
-        if (!kWrite) {
+        if (!kWrite || (kClip && op >= lim)) {
             op += total;
             base = nbase;
             continue;
         }
-        // ---- execute
+        // ---- execute (xlen: the bytes of the element that are written)
+        const u32 xlen = kClip ? (dst >= lim ? 0u : min(elen, lim - dst)) : elen;
         const u32 lsrc = p + hdr;  // literal bytes start behind the header
         // highest output byte (exclusive) the element reads; literals read none
-        const u32 need = (mine && is_copy) ? (dst - eoff + min(elen, eoff)) : 0u;
-        u32 pending = R;
+        const u32 need = (mine && is_copy) ? (dst - eoff + min(xlen, eoff)) : 0u;
+        u32 pending = kClip ? __ballot_sync(kFullMask, xlen != 0u) : R;
         while (pending) {
             const u32 f = (u32)__ffs((int)pending) - 1u;
             const u32 frontier = __shfl_sync(kFullMask, dst, f);
-            const u32 flen = __shfl_sync(kFullMask, elen, f);
+            const u32 flen = __shfl_sync(kFullMask, xlen, f);
             if (flen > kShortElem) {
                 const u32 fcopy = __shfl_sync(kFullMask, (u32)is_copy, f);
                 const u32 fx = __shfl_sync(kFullMask, is_copy ? eoff : lsrc, f);
@@ -317,12 +322,12 @@ __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 
                 pending &= ~(1u << f);
                 continue;
             }
-            const bool ready = ((pending >> lane) & 1u) && elen <= kShortElem && need <= frontier;
+            const bool ready = ((pending >> lane) & 1u) && xlen <= kShortElem && need <= frontier;
             if (ready) {
                 u8* d = o + dst;
-                if (is_copy && eoff < elen) {
+                if (is_copy && eoff < xlen) {
                     const u8* s = o + (dst - eoff);
-                    for (u32 i = 0, k = 0; i < elen; i++) {  // pattern of `offset` bytes repeats
+                    for (u32 i = 0, k = 0; i < xlen; i++) {  // pattern of `offset` bytes repeats
                         d[i] = s[k];
                         k = (k + 1 == eoff) ? 0 : k + 1;
                     }
@@ -332,7 +337,7 @@ __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 
                     const uintptr_t sa = reinterpret_cast<uintptr_t>(is_copy ? o + (dst - eoff) : src + lsrc);
                     const u32* w = reinterpret_cast<const u32*>(sa & ~(uintptr_t)3);
                     const u32 sh = (u32)sa << 3;
-                    const u32 last = (((u32)sa & 3u) + elen - 1u) >> 2;  // index of the last word needed (0..4)
+                    const u32 last = (((u32)sa & 3u) + xlen - 1u) >> 2;  // index of the last word needed (0..4)
                     u32 w0, w1 = 0, w2 = 0, w3 = 0, w4 = 0;
                     if (is_copy) {  // output bytes written earlier in this kernel: coherent loads
                         w0 = w[0];
@@ -352,7 +357,7 @@ __device__ __forceinline__ bool decode_fast_warp(const u8* __restrict__ in, u64 
 #pragma unroll
                     for (u32 i = 0; i < 16; i++) {
                         const u32 word = i < 4 ? b0 : (i < 8 ? b1 : (i < 12 ? b2 : b3));
-                        if (i < elen) d[i] = (u8)(word >> (8 * (i & 3)));
+                        if (i < xlen) d[i] = (u8)(word >> (8 * (i & 3)));
                     }
                 }
             }
@@ -442,6 +447,111 @@ k_validate_fragments(const u8* __restrict__ in, const u64* __restrict__ frag_off
               (oe >= ob);
     if (ok) ok = decode_fast_warp<false>(in, ip, ie, nullptr, on, lane);
     if (!ok && lane == 0) atomicOr(&res->fallback, 1u);
+}
+
+// Range decoding (snappy_b200_uncompress_range*_device): bytes [offset, offset + length) of a stream's output, from the
+// tiles t0 .. t0 + (number of work items) - 1 that overlap it.  Tile f is in[frag_off[f] .. frag_off[f+1]) and
+// produces output bytes [out_start[f], out_start[f+1]) (out_start null: the 64 KiB fragments of a side index).
+struct RangeDesc {
+    const u8* in;
+    const u64* frag_off;
+    const u64* out_start;
+    u8* out;               // receives [offset, offset + length)
+    u64 in_begin, in_end;  // the element bytes of the stream: in[in_begin .. in_end)
+    u64 out_len;           // the claimed length
+    u64 offset, length;
+    u32 nfrag, t0;
+    u32 work_begin;        // the request's first work item; requests are in work order
+    u32 pad;
+};
+
+constexpr u32 kRangeCtasPerSm = 16;  // persistent CTAs per SM of k_decode_range: 32 warps, one scratch slot each
+
+// One warp per (request, tile) work item, persistent warps pulling items from *next_work.  Every tile gets the
+// per-fragment checks of k_decode_fragments over its whole length, and only its bytes inside the range are written:
+//   interior (the tile lies inside the range): the full decode straight into the destination;
+//   trailing edge (the tile starts inside the range and ends behind it): the clipped decode into the destination;
+//   leading edge (the range starts inside the tile): the clipped decode up to the range end into the warp's scratch
+//   slot (slots + warp * slot_stride; slot_stride 0 when one request has at most one such tile), then the wanted part.
+// A tile that is not clean raises flags[request] and res->fallback; the host then takes the index-free chain.
+__global__ void __launch_bounds__(kDecodeWarpsPerCta * 32, kRangeCtasPerSm)
+k_decode_range(const RangeDesc* __restrict__ descs, u32 ndesc, u32 nwork, u32* __restrict__ next_work,
+               u8* __restrict__ slots, u64 slot_stride, u32* __restrict__ flags, DecodeResult* __restrict__ res) {
+    const u32 lane = lane_id();
+    const u32 warp = blockIdx.x * kDecodeWarpsPerCta + (threadIdx.x >> 5);
+    u8* slot = slots + warp * slot_stride;
+    for (;;) {
+        u32 w = 0;
+        if (lane == 0) w = atomicAdd(next_work, 1u);
+        w = __shfl_sync(kFullMask, w, 0);
+        if (w >= nwork) return;
+        u32 lo = 0, hi = ndesc;  // the request: descs[lo].work_begin <= w < descs[lo + 1].work_begin
+        while (hi - lo > 1) {
+            const u32 mid = lo + ((hi - lo) >> 1);
+            if (descs[mid].work_begin <= w) lo = mid;
+            else hi = mid;
+        }
+        const RangeDesc& d = descs[lo];
+        const u32 f = d.t0 + (w - d.work_begin);
+        const u64 ip = d.frag_off[f];
+        const u64 ie = d.frag_off[f + 1];
+        const u64 ob = d.out_start ? d.out_start[f] : (u64)f * kBlockSize;
+        u64 oe = d.out_start ? d.out_start[f + 1] : ob + kBlockSize;
+        if (oe > d.out_len) oe = d.out_len;
+        const u32 on = (oe >= ob && oe - ob <= 0xffffffffull) ? (u32)(oe - ob) : 0u;
+        const u64 end = d.offset + d.length;
+        bool ok = (ie >= ip) && (ie <= d.in_end) && (f != 0 || ip == d.in_begin) && (f != d.nfrag - 1 || ie == d.in_end) &&
+                  (oe >= ob) && (ob <= d.out_len) && (oe > d.offset || on == 0) && (ob < end || on == 0);
+        if (ok && on) {
+            if (ob < d.offset) {
+                const u32 lim = (u32)((oe < end ? oe : end) - ob);
+                ok = decode_fast_warp<true, true>(d.in, ip, ie, slot, on, lane, lim);
+                __syncwarp();
+                if (ok) warp_copy_forward<false>(d.out, slot + (d.offset - ob), lim - (d.offset - ob), lane);
+            } else if (oe > end) {
+                ok = decode_fast_warp<true, true>(d.in, ip, ie, d.out + (ob - d.offset), on, lane, (u32)(end - ob));
+            } else {
+                ok = decode_fast_warp(d.in, ip, ie, d.out + (ob - d.offset), on, lane);
+            }
+        }
+        __syncwarp();
+        if (!ok && lane == 0) {
+            atomicOr(&flags[lo], 1u);
+            atomicOr(&res->fallback, 1u);
+        }
+    }
+}
+
+// The tiles of the parse's index (out_start, monotone, out_start[nfrag] = claimed) that overlap [offset, end), end >
+// offset: t0 / t1 = the last tile starting at or below offset / end - 1, and the bytes of tile t0 below end (the scratch
+// slot a leading edge needs; 0 when tile t0 starts at offset).  One thread.
+__global__ void k_range_tiles(const u64* __restrict__ out_start, u32 nfrag, u64 offset, u64 end, u64* __restrict__ out3) {
+    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    u32 t[2];
+    const u64 x[2] = {offset, end - 1};
+    for (int k = 0; k < 2; k++) {
+        u32 lo = 0, hi = nfrag;  // out_start[lo] <= x < out_start[hi]
+        while (hi - lo > 1) {
+            const u32 mid = lo + ((hi - lo) >> 1);
+            if (out_start[mid] <= x[k]) lo = mid;
+            else hi = mid;
+        }
+        t[k] = lo;
+    }
+    const u64 ob = out_start[t[0]], oe = out_start[t[0] + 1];
+    out3[0] = t[0];
+    out3[1] = t[1];
+    out3[2] = ob < offset ? (oe < end ? oe : end) - ob : 0;
+}
+
+// The first (up to) 5 bytes of every request's stream, for the host's varint parse: hb[8 i + k], byte 5 = how many.
+__global__ void __launch_bounds__(256)
+k_range_headers(const u8* const* __restrict__ ins, const u64* __restrict__ lens, u32 count, u8* __restrict__ hb) {
+    const u32 i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= count) return;
+    const u32 n = lens[i] < 5 ? (u32)lens[i] : 5u;
+    for (u32 k = 0; k < 5; k++) hb[8 * (u64)i + k] = k < n ? ins[i][k] : 0;
+    hb[8 * (u64)i + 5] = (u8)n;
 }
 
 // Status arbiter, bounded: only the tiles the parallel decoder rejected (tile_flags) are decoded again, one warp,

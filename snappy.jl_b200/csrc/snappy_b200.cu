@@ -122,6 +122,8 @@ struct Context {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     // scratch for decode
     DevBuf result, parse_a, parse_b, parse_c, parse_d, index, index_out, tile_flags;
+    // scratch for range decoding: request descriptors + flags, leading-edge slots, the whole output of paths 2-3
+    DevBuf range_desc, range_slots, range_full;
     // staging for the host-buffer API
     DevBuf stage_in, stage_out;
     void* pinned = nullptr;  // small pinned readback area (kPinnedBytes)
@@ -414,7 +416,8 @@ void ctx_destroy(Context& c) {
     if (c.ev_join) cudaEventDestroy(c.ev_join);
     c.ev_fork = c.ev_join = nullptr;
     for (DevBuf* b : {&c.descs, &c.tail, &c.gtables, &c.scratch, &c.frag_sizes, &c.frag_offsets, &c.result, &c.parse_a,
-                      &c.parse_b, &c.parse_c, &c.parse_d, &c.index, &c.stage_in, &c.stage_out, &c.flags, &c.order, &c.trace, &c.index_out, &c.tile_flags})
+                      &c.parse_b, &c.parse_c, &c.parse_d, &c.index, &c.stage_in, &c.stage_out, &c.flags, &c.order, &c.trace, &c.index_out, &c.tile_flags,
+                      &c.range_desc, &c.range_slots, &c.range_full})
         b->release();
     if (c.pinned) cudaFreeHost(c.pinned);
     if (c.pinned_zero) cudaFreeHost(c.pinned_zero);
@@ -1018,14 +1021,18 @@ int build_index_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 cla
     return total == claimed ? 0 : -1;
 }
 
-// Arbitrary stream, no usable side index.  The parse builds the tile index (relaxed: a literal may straddle a 64 KiB
-// boundary); the indexed decoder runs over every tile whose both ends are known and marks the tiles it rejects; the
-// bounded serial walk (k_decode_serial_tiles) then decodes only those, and everything behind the point where the
-// parse lost the chain, with the reference's checks.  So a corrupt 1 GiB stream costs the parallel decode of its good
-// prefix plus one tile of serial work, and the status is the reference's.  Returns a status (>= 0), or -1: nothing
-// usable came out of the parse (caller: whole-stream serial decoder).
-int decode_parsed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u8* d_out, u32 claimed, cudaStream_t st,
-                         u8* host_out, bool* host_copied) {
+// The parse-and-tile set-up of the index-free decode (decode_parsed_locked, range decoding): the relaxed parse builds
+// the tile index (c.index: tile starts in the stream, c.index_out: their output positions; a literal may straddle a
+// 64 KiB boundary), clean cuts re-tile a complete parse whose copies cross the boundaries, and tiles [0, tvalid) have
+// both ends in the index.  Returns 0 when the tiles are set up, a status (> 0) when the parse alone decides (its first
+// failing element, or an error-free parse whose lengths do not add up: path 1) or a CUDA call failed, and -1 when nothing
+// usable came out of the parse.
+struct ParsedTiles {
+    u64 pflags = 0;
+    bool complete = false;  // the parse followed the chain to the end without an error and the lengths add up
+    u32 tvalid = 0;
+};
+int parse_tiles_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, cudaStream_t st, ParsedTiles& P) {
     const u32 nfrag = frag_count(claimed);
     if (nfrag == 0 || n <= hdr) return -1;
     CU(c.index.ensure(((size_t)nfrag + 1) * 8));
@@ -1093,6 +1100,30 @@ int decode_parsed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u8* d
         tvalid = first == 0 ? 0u : (first > nfrag ? nfrag : first - 1);
         if (first <= nfrag && first > 0 && tvalid > 0) tvalid = first - 1;
     }
+    P.pflags = pflags;
+    P.complete = complete;
+    P.tvalid = tvalid;
+    return 0;
+}
+
+// Arbitrary stream, no usable side index.  The parse builds the tile index (parse_tiles_locked); the indexed decoder
+// runs over every tile whose both ends are known and marks the tiles it rejects; the bounded serial walk
+// (k_decode_serial_tiles) then decodes only those, and everything behind the point where the parse lost the chain,
+// with the reference's checks.  So a corrupt 1 GiB stream costs the parallel decode of its good prefix plus one tile of
+// serial work, and the status is the reference's.  Returns a status (>= 0), or -1: nothing usable came out of the
+// parse (caller: whole-stream serial decoder).
+int decode_parsed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u8* d_out, u32 claimed, cudaStream_t st,
+                         u8* host_out, bool* host_copied) {
+    const u32 nfrag = frag_count(claimed);
+    ParsedTiles P;
+    int rc = parse_tiles_locked(c, d_in, n, hdr, claimed, st, P);
+    if (rc != 0) return rc;
+    u64* idx = (u64*)c.index.p;
+    u64* ost = (u64*)c.index_out.p;
+    u8* tf = (u8*)c.tile_flags.p;
+    const u64 pflags = P.pflags;
+    const bool complete = P.complete;
+    const u32 tvalid = P.tvalid;
     CU(cudaMemsetAsync(c.result.p, 0, sizeof(DecodeResult), st));
     if (c.opt.timing) CU(cudaEventRecord(c.ev[2], st));
     // host-buffer API: ranged device-to-host copies only when the tiles are the aligned 64 KiB fragments
@@ -1268,6 +1299,265 @@ int validate_device_locked(Context& c, const u8* d_in, size_t n, const u64* d_in
     }
     c.last_path = 3;
     return validate_exact_locked(c, d_in, n, hdr, claimed, st);
+}
+
+// ---- range decoding (snappy_b200_uncompress_range*_device) ------------------------------------------------------
+// Bytes [offset, offset + length) of what uncompress writes, decoding only the tiles that overlap them.
+//   path 0: a side index; one k_decode_range launch over fragments offset / 64 KiB .. (end - 1) / 64 KiB.  If every one
+//           of them is clean, that is the answer (the index is trusted for where they start); otherwise path 1.
+//   path 1: the index-free parse (parse_tiles_locked) decides the status, or shows the stream valid; then one launch
+//           over the parse's tiles that overlap the range.
+//   paths 2-3: the parse lost the chain, or a touched tile was rejected: validation gives the status, and only a valid
+//           stream is decoded whole into c.range_full to copy the range out (2: the parse took part, 3: whole-stream
+//           serial walk only).  This is the only path whose device memory is O(claimed).
+
+// the header of the stream in d_in[0 .. n): BAD_VARINT or OK
+int read_header_locked(Context& c, const u8* d_in, size_t n, u32* claimed, size_t* hdr, cudaStream_t st) {
+    u8* hb = (u8*)c.pinned + 256;
+    const size_t hn = n < 5 ? n : 5;
+    if (hn) {
+        CU(cudaMemcpyAsync(hb, d_in, hn, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+    }
+    return parse_varint(hb, hn, claimed, hdr);
+}
+
+// One persistent k_decode_range launch over the ndesc requests in c.range_desc (descriptors, then one u32 flag per
+// request, zeroed here).  slot_stride 0: at most one leading-edge tile in the launch, slot_bytes of scratch; else one
+// slot of slot_stride bytes per launched warp (every warp of the grid pulls work, so a grid rounded up to whole CTAs
+// needs a slot for each).  Returns OK, or -1 when some tile was not clean (flags say whose).
+int range_launch(Context& c, u32 ndesc, u32 nwork, u64 slot_bytes, u64 slot_stride, cudaStream_t st) {
+    const RangeDesc* descs = (const RangeDesc*)c.range_desc.p;
+    u32* flags = (u32*)((u8*)c.range_desc.p + (size_t)ndesc * sizeof(RangeDesc));
+    const u32 cap = (u32)c.sm_count * kRangeCtasPerSm * kDecodeWarpsPerCta;
+    const u32 grid = ((nwork < cap ? nwork : cap) + kDecodeWarpsPerCta - 1) / kDecodeWarpsPerCta;
+    const size_t warps = (size_t)grid * kDecodeWarpsPerCta;
+    CU(c.range_slots.ensure((slot_stride ? warps * slot_stride : (size_t)slot_bytes) + 64));
+    u32* next_work = (u32*)((u8*)c.result.p + 192);
+    CU(cudaMemsetAsync(flags, 0, (size_t)ndesc * 4, st));
+    CU(cudaMemsetAsync(next_work, 0, 4, st));
+    CU(cudaMemsetAsync(c.result.p, 0, sizeof(DecodeResult), st));
+    if (c.opt.timing) CU(cudaEventRecord(c.ev[2], st));
+    k_decode_range<<<grid, kDecodeWarpsPerCta * 32, 0, st>>>(
+        descs, ndesc, nwork, next_work, (u8*)c.range_slots.p, slot_stride, flags, (DecodeResult*)c.result.p);
+    c.last_launches[1] += 1;
+    return decode_finish(c, st, false);
+}
+
+// one request as the only descriptor of c.range_desc
+int range_put_one(Context& c, const RangeDesc& d, cudaStream_t st) {
+    CU(c.range_desc.ensure(sizeof(RangeDesc) + 4));
+    RangeDesc* h = (RangeDesc*)((u8*)c.pinned + 4096);
+    *h = d;
+    CU(cudaMemcpyAsync(c.range_desc.p, h, sizeof(RangeDesc), cudaMemcpyHostToDevice, st));
+    return SNAPPY_B200_OK;
+}
+
+RangeDesc range_desc(const u8* d_in, size_t n, size_t hdr, u32 claimed, u64 offset, size_t length, u8* d_out) {
+    RangeDesc d{};
+    d.in = d_in;
+    d.out = d_out;
+    d.in_begin = hdr;
+    d.in_end = n;
+    d.out_len = claimed;
+    d.offset = offset;
+    d.length = length;
+    d.nfrag = frag_count(claimed);
+    return d;
+}
+
+// path 0 for one request: OK, or -1 when a touched fragment is not clean (length > 0)
+int range_indexed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, const u64* d_index, u64 offset,
+                         size_t length, u8* d_out, cudaStream_t st) {
+    const u64 end = offset + length;
+    RangeDesc d = range_desc(d_in, n, hdr, claimed, offset, length, d_out);
+    d.frag_off = d_index;
+    d.t0 = (u32)(offset / kBlockSize);
+    const u32 t1 = (u32)((end - 1) / kBlockSize);
+    const u64 ob = (u64)d.t0 * kBlockSize;
+    const u64 oe = ob + kBlockSize < end ? ob + kBlockSize : end;
+    int rc = range_put_one(c, d, st);
+    if (rc != SNAPPY_B200_OK) return rc;
+    return range_launch(c, 1, t1 - d.t0 + 1, ob < offset ? oe - ob : 0, 0, st);
+}
+
+// path 1: a status (>= 0), or -1 (caller: paths 2-3; *valid when the parse showed the stream valid)
+int range_parsed_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, u64 offset, size_t length,
+                        u8* d_out, cudaStream_t st, bool* valid) {
+    ParsedTiles P;
+    int rc = parse_tiles_locked(c, d_in, n, hdr, claimed, st, P);
+    if (rc != 0) return rc;
+    if (!P.complete) return -1;
+    *valid = true;  // a complete, error-free parse whose lengths add up (validate_parsed_locked)
+    c.last_path = 1;
+    if (length == 0) return SNAPPY_B200_OK;
+    u64* d3 = (u64*)((u8*)c.result.p + 160);
+    u64* h3 = (u64*)((u8*)c.pinned + 4096 + 512);
+    k_range_tiles<<<1, 32, 0, st>>>((const u64*)c.index_out.p, frag_count(claimed), offset, offset + length, d3);
+    c.last_launches[1] += 1;
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h3, d3, 24, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    RangeDesc d = range_desc(d_in, n, hdr, claimed, offset, length, d_out);
+    d.frag_off = (const u64*)c.index.p;
+    d.out_start = (const u64*)c.index_out.p;
+    d.t0 = (u32)h3[0];
+    const u32 t1 = (u32)h3[1];
+    const u64 slot = h3[2];
+    rc = range_put_one(c, d, st);
+    if (rc != SNAPPY_B200_OK) return rc;
+    return range_launch(c, 1, t1 - d.t0 + 1, slot, 0, st);
+}
+
+// paths 2-3: validation for the status (skipped when the parse showed the stream valid), then a whole decode of the
+// valid stream into context scratch and the copy of the range
+int range_whole_locked(Context& c, const u8* d_in, size_t n, u32 claimed, u64 offset, size_t length, u8* d_out,
+                       cudaStream_t st, bool valid) {
+    int launches = c.last_launches[1];
+    int rc = SNAPPY_B200_OK;
+    if (!valid) {
+        rc = validate_device_locked(c, d_in, n, nullptr, nullptr, st);
+        launches += c.last_launches[1];
+    }
+    if (rc == SNAPPY_B200_OK) {
+        size_t out_len = 0;
+        rc = c.range_full.ensure((size_t)claimed + 64) == cudaSuccess ? SNAPPY_B200_OK
+                                                                       : fail_cuda(cudaErrorMemoryAllocation, "range_full");
+        if (rc == SNAPPY_B200_OK) {
+            rc = uncompress_device_locked(c, d_in, n, (u8*)c.range_full.p, claimed, &out_len, nullptr, st);
+            launches += c.last_launches[1];
+        }
+        if (rc == SNAPPY_B200_OK && length) {
+            CU(cudaMemcpyAsync(d_out, (u8*)c.range_full.p + offset, length, cudaMemcpyDeviceToDevice, st));
+            CU(cudaStreamSynchronize(st));
+        }
+    }
+    c.last_launches[1] = launches;
+    c.last_path = c.last_path == 3 ? 3 : 2;
+    return rc;
+}
+
+// everything after the header and range checks; d_index may be null
+int range_chain_locked(Context& c, const u8* d_in, size_t n, size_t hdr, u32 claimed, const u64* d_index, u64 offset,
+                       size_t length, u8* d_out, cudaStream_t st) {
+    bool valid = false;
+    if (c.opt.decode_variant != 1) {
+        if (d_index) {  // trusted for where the touched fragments start; any of them not clean: the index-free chain
+            c.last_path = 0;
+            if (length == 0) return SNAPPY_B200_OK;
+            const int rc = range_indexed_locked(c, d_in, n, hdr, claimed, d_index, offset, length, d_out, st);
+            if (rc >= 0) return rc;
+        }
+        const int rc = range_parsed_locked(c, d_in, n, hdr, claimed, offset, length, d_out, st, &valid);
+        if (rc >= 0) return rc;
+    }
+    c.last_path = 3;
+    return range_whole_locked(c, d_in, n, claimed, offset, length, d_out, st, valid);
+}
+
+int uncompress_range_locked(Context& c, const u8* d_in, size_t n, const u64* d_index, u64 offset, size_t length,
+                            u8* d_out, cudaStream_t st) {
+    c.last_launches[1] = 0;
+    u32 claimed = 0;
+    size_t hdr = 0;
+    const int rc = read_header_locked(c, d_in, n, &claimed, &hdr, st);
+    if (rc != SNAPPY_B200_OK) return rc;
+    if (offset > claimed || length > claimed - offset) return SNAPPY_B200_BAD_ARGUMENT;
+    return range_chain_locked(c, d_in, n, hdr, claimed, d_index, offset, length, d_out, st);
+}
+
+// The batched call: every header through one kernel and one copy, one k_decode_range launch over the (request,
+// fragment) work of every request that has an index, then the single-range chain (without the index) for each request
+// that has none or had a fragment rejected.
+int uncompress_ranges_locked(Context& c, const u8* const* d_ins, const size_t* in_lens,
+                             const uint64_t* const* d_indexes, const uint64_t* offsets, const size_t* lengths,
+                             uint8_t* const* d_outs, size_t count, int* statuses, cudaStream_t st) {
+    c.last_launches[1] = 0;
+    if (count == 0) return SNAPPY_B200_OK;
+    if (count > 0x7fffffffull) return SNAPPY_B200_BAD_ARGUMENT;
+    // ---- the headers
+    std::vector<u64> lens(count);
+    for (size_t i = 0; i < count; i++) lens[i] = d_ins[i] ? in_lens[i] : 0;  // a null stream is BAD_ARGUMENT below
+    const size_t hb_off = count * 16;
+    CU(c.range_desc.ensure(hb_off + count * 8));
+    u8* dbuf = (u8*)c.range_desc.p;
+    CU(cudaMemcpyAsync(dbuf, d_ins, count * 8, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dbuf + count * 8, lens.data(), count * 8, cudaMemcpyHostToDevice, st));
+    k_range_headers<<<(u32)((count + 255) / 256), 256, 0, st>>>((const u8* const*)dbuf, (const u64*)(dbuf + count * 8),
+                                                                (u32)count, dbuf + hb_off);
+    CU(cudaGetLastError());
+    std::vector<u8> hb(count * 8);
+    CU(cudaMemcpyAsync(hb.data(), dbuf + hb_off, count * 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    // ---- the work list
+    std::vector<u32> claimed(count, 0);
+    std::vector<size_t> hdrs(count, 0);
+    std::vector<RangeDesc> descs;
+    std::vector<size_t> req;   // request of each descriptor
+    std::vector<size_t> rest;  // requests for the single-range chain
+    u64 nwork = 0;
+    for (size_t i = 0; i < count; i++) {
+        const u64 off = offsets[i];
+        const size_t len = lengths[i];
+        if ((!d_ins[i] && in_lens[i]) || (!d_outs[i] && len)) {
+            statuses[i] = SNAPPY_B200_BAD_ARGUMENT;
+            continue;
+        }
+        statuses[i] = parse_varint(&hb[8 * i], hb[8 * i + 5], &claimed[i], &hdrs[i]);
+        if (statuses[i] != SNAPPY_B200_OK) continue;
+        if (off > claimed[i] || len > claimed[i] - off) {
+            statuses[i] = SNAPPY_B200_BAD_ARGUMENT;
+            continue;
+        }
+        const u64* idx = d_indexes ? (const u64*)d_indexes[i] : nullptr;
+        if (!idx || c.opt.decode_variant == 1) {
+            rest.push_back(i);
+            continue;
+        }
+        if (len == 0) continue;  // path 0 touches no fragment
+        RangeDesc d = range_desc(d_ins[i], in_lens[i], hdrs[i], claimed[i], off, len, d_outs[i]);
+        d.frag_off = idx;
+        d.t0 = (u32)(off / kBlockSize);
+        d.work_begin = (u32)nwork;
+        nwork += (u64)((off + len - 1) / kBlockSize) - d.t0 + 1;
+        // the launch numbers its work items with a 32-bit counter that every warp moves once past the last one
+        if (nwork > 0x7fffffffull) return SNAPPY_B200_BAD_ARGUMENT;
+        descs.push_back(d);
+        req.push_back(i);
+    }
+    // ---- one launch for the indexed requests
+    int path = 0;
+    float ms = 0.f;
+    if (!descs.empty()) {
+        const size_t nd = descs.size();
+        CU(c.range_desc.ensure(nd * (sizeof(RangeDesc) + 4)));
+        CU(cudaMemcpyAsync(c.range_desc.p, descs.data(), nd * sizeof(RangeDesc), cudaMemcpyHostToDevice, st));
+        const int rc = range_launch(c, (u32)nd, (u32)nwork, 0, kBlockSize, st);
+        if (rc > 0) return rc;
+        ms = c.last_ms[1];
+        if (rc < 0) {  // some fragment was not clean: those requests go on as if they had no index
+            std::vector<u32> flags(nd);
+            CU(cudaMemcpyAsync(flags.data(), (u8*)c.range_desc.p + nd * sizeof(RangeDesc), nd * 4, cudaMemcpyDeviceToHost,
+                               st));
+            CU(cudaStreamSynchronize(st));
+            for (size_t k = 0; k < nd; k++)
+                if (flags[k]) rest.push_back(req[k]);
+        }
+    }
+    // ---- the rest, one at a time
+    int launches = c.last_launches[1];
+    for (size_t i : rest) {
+        c.last_launches[1] = 0;
+        statuses[i] = range_chain_locked(c, d_ins[i], in_lens[i], hdrs[i], claimed[i], nullptr, offsets[i], lengths[i],
+                                         d_outs[i], st);
+        launches += c.last_launches[1];
+        path = c.last_path > path ? c.last_path : path;
+        if (statuses[i] == SNAPPY_B200_CUDA_ERROR) return statuses[i];
+    }
+    c.last_launches[1] = launches;
+    c.last_path = path;
+    c.last_ms[1] = ms;
+    return SNAPPY_B200_OK;
 }
 
 // Takes a lane of the addressed device for the duration of a call: resolves the device, makes it current (the
@@ -1456,6 +1746,26 @@ int snappy_b200_validate_device(const uint8_t* d_in, size_t n, const uint64_t* d
     Locked L;
     if (L.rc != SNAPPY_B200_OK) return L.rc;
     return validate_device_locked(*L.c, d_in, n, (const u64*)d_frag_index, uncompressed_len, (cudaStream_t)stream);
+}
+
+int snappy_b200_uncompress_range_device(const uint8_t* d_in, size_t n, const uint64_t* d_frag_index, uint64_t offset,
+                                        size_t length, uint8_t* d_out, void* stream) {
+    if ((!d_in && n) || (!d_out && length)) return SNAPPY_B200_BAD_ARGUMENT;
+    Locked L;
+    if (L.rc != SNAPPY_B200_OK) return L.rc;
+    return uncompress_range_locked(*L.c, d_in, n, (const u64*)d_frag_index, offset, length, d_out,
+                                   (cudaStream_t)stream);
+}
+
+int snappy_b200_uncompress_ranges_device(const uint8_t* const* d_ins, const size_t* in_lens,
+                                         const uint64_t* const* d_frag_indexes, const uint64_t* offsets,
+                                         const size_t* lengths, uint8_t* const* d_outs, size_t count, int* statuses,
+                                         void* stream) {
+    if (count && (!d_ins || !in_lens || !offsets || !lengths || !d_outs || !statuses)) return SNAPPY_B200_BAD_ARGUMENT;
+    Locked L;
+    if (L.rc != SNAPPY_B200_OK) return L.rc;
+    return uncompress_ranges_locked(*L.c, d_ins, in_lens, d_frag_indexes, offsets, lengths, d_outs, count, statuses,
+                                    (cudaStream_t)stream);
 }
 
 extern "C++" {

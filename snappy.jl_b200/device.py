@@ -86,6 +86,100 @@ def validate_device(stream, index=None):
     return rc, (None if rc == _abi.BAD_VARINT else claimed.value)
 
 
+def _claimed_lengths(streams):
+    """the header's claimed length of each stream (None where it does not parse), one device-to-host copy for all
+    distinct streams"""
+    from .api import parse32
+    distinct = {}
+    for t in streams:
+        distinct.setdefault(t.data_ptr(), t)
+    keys = list(distinct)
+    heads = torch.zeros((len(keys), 5), dtype=torch.uint8, device=streams[0].device)
+    for k, key in enumerate(keys):
+        t = distinct[key]
+        heads[k, : min(5, t.numel())] = t[:5]
+    heads = heads.cpu().numpy()
+    claimed = {}
+    for k, key in enumerate(keys):
+        try:
+            claimed[key] = parse32(heads[k, : min(5, distinct[key].numel())], 0)[0]
+        except SnappyError:
+            claimed[key] = None
+    return [claimed[t.data_ptr()] for t in streams]
+
+
+def _check_range_args(stream, index, claimed):
+    if stream.dtype != torch.uint8 or not stream.is_cuda or not stream.is_contiguous():
+        raise ValueError("stream: expected a contiguous uint8 CUDA tensor")
+    if index is None:
+        return
+    if index.dtype not in (torch.int64, torch.uint64) or not index.is_cuda or not index.is_contiguous() or \
+            index.device != stream.device:
+        raise ValueError("index: expected a contiguous int64 CUDA tensor on the stream's device")
+    if claimed is not None and index.numel() < nfragments(claimed) + 1:
+        raise ValueError("index has %d entries; the stream claims %d bytes, which needs %d"
+                         % (index.numel(), claimed, nfragments(claimed) + 1))
+
+
+def uncompress_range_device(stream, offset, length, index=None, out=None):
+    """Bytes [offset, offset + length) of uncompress_device(stream), decoding only the tiles that overlap them.
+
+    Without `index` the result (bytes, or the SnappyError raised) is exactly what uncompress_device gives, sliced.
+    With `index` (the side index of compress_device, (nfrag + 1) x int64) the call trusts it for where the touched
+    64 KiB fragments start: if they all decode cleanly the bytes are returned without looking at the rest of the
+    stream; otherwise the call proceeds as without the index.  `out` may be a preallocated contiguous uint8 tensor on
+    the stream's device with at least `length` bytes; nothing outside its first `length` bytes is written."""
+    _check_range_args(stream, index, _claimed_lengths([stream])[0] if index is not None else None)
+    if out is None:
+        out = torch.empty(length, dtype=torch.uint8, device=stream.device)
+    elif out.dtype != torch.uint8 or out.device != stream.device or not out.is_contiguous():
+        raise ValueError("out: expected a contiguous uint8 tensor on the stream's device")
+    elif out.numel() < length:
+        raise SnappyError(_abi.BUFFER_TOO_SMALL)
+    with torch.cuda.device(stream.device):
+        _abi.lib().snappy_b200_init(stream.device.index)
+        _check(_abi.lib().snappy_b200_uncompress_range_device(
+            _dev_ptr(stream), stream.numel(), _dev_ptr(index), int(offset), int(length), _dev_ptr(out),
+            _stream_ptr(stream.device)))
+    return out[:length]
+
+
+def uncompress_ranges_device(streams, offsets, lengths, indexes=None):
+    """Batched uncompress_range_device: request i reads [offsets[i], offsets[i] + lengths[i]) of streams[i] (the same
+    tensor may appear many times), with indexes[i] (None: no index).  Returns (list of tensors, statuses): per request
+    the bytes -- views into one buffer -- and what uncompress_range_device would report (0 or a status; the bytes are
+    undefined unless the status is 0)."""
+    count = len(streams)
+    if not (len(offsets) == len(lengths) == count) or (indexes is not None and len(indexes) != count):
+        raise ValueError("streams, offsets, lengths and indexes must have one entry per request")
+    if count == 0:
+        return [], []
+    dev = streams[0].device
+    pairs = {(id(t), id(i)): (t, i) for t, i in zip(streams, indexes if indexes is not None else [None] * count)}
+    pairs = list(pairs.values())
+    claimed = _claimed_lengths([t for t, i in pairs]) if any(i is not None for _, i in pairs) else [None] * len(pairs)
+    for (t, i), c in zip(pairs, claimed):
+        if t.device != dev:
+            raise ValueError("expected every stream on one device")
+        _check_range_args(t, i, c)
+    lens_py = [int(n) for n in lengths]
+    flat = torch.empty(max(sum(lens_py), 1), dtype=torch.uint8, device=dev)
+    base, starts, o = flat.data_ptr(), [], 0
+    for n in lens_py:
+        starts.append(base + o)
+        o += n
+    in_lens = (ctypes.c_size_t * count)(*[s.numel() for s in streams])
+    offs = (ctypes.c_uint64 * count)(*[int(o) for o in offsets])
+    lens = (ctypes.c_size_t * count)(*lens_py)
+    statuses = (ctypes.c_int * count)()
+    with torch.cuda.device(dev):
+        _abi.lib().snappy_b200_init(dev.index)
+        _check(_abi.lib().snappy_b200_uncompress_ranges_device(
+            _ptr_array(streams), in_lens, _ptr_array(indexes) if indexes is not None else None, offs, lens,
+            (ctypes.c_void_p * count)(*starts), count, statuses, _stream_ptr(dev)))
+    return list(flat[: sum(lens_py)].split(lens_py)), list(statuses)
+
+
 def compress_shard_device(shard, total_len, out=None, want_sizes=False):
     """Compress a run of whole fragments of a stream whose total length is `total_len`
     (elements only, no varint header).  Returns (bytes_view, frag_sizes or None)."""

@@ -26,8 +26,10 @@
 //     and "0 mismatches" when both statuses equal the oracle's.
 //   mode "validate-pages": every stream as one page of ONE k_validate_pages launch (no output), plus two empty pages.
 //     Per page: status and claimed length against the oracle.
+//   mode "range": uncompress_range_locked (snappy_b200.cu), kernel for kernel, for the ranges listed in F.ranges, with
+//     the side index F<IDX_SUFFIX> when it exists; see run_range.
 //   g++ -O1 -std=c++17 -DSB200_CPU_EMU -Itools/cpu_warp tools/cpu_warp/run_decode_parsed.cpp oracle.o
-//   ./a.out parsed|pages|validate|validate-pages file...
+//   ./a.out parsed|pages|validate|validate-pages|range file...
 #include "../../snappy.jl_b200/csrc/parse.cuh"
 
 #include <string>
@@ -45,6 +47,12 @@ using cpu_warp::launch_independent_threads;
 
 constexpr u8 kSentinel = 0xEE;
 constexpr size_t kGuard = 256;  // sentinel bytes behind every output
+
+static bool sentinels_intact(const u8* p, size_t len) {
+    for (size_t i = 0; i < len; i++)
+        if (p[i] != kSentinel) return false;
+    return true;
+}
 
 static void as_warp(u32 block, u32 tid_base, u32 block_dim) {
     cpu_warp::W().block = block;
@@ -201,17 +209,11 @@ static u32 tiles_valid(const std::vector<u64>& idx, u32 nfrag, u64 n) {
     return tvalid;
 }
 
-static int decode_parsed(const u8* in, u64 n, u64 hdr, u32 claimed, u8* out, u32 pshift, bool clean_cuts, int* path) {
+// parse_tiles_locked (snappy_b200.cu): the parse, its verdicts (path 1: a status > 0), clean cuts, tvalid; 0 when the
+// tiles are set up
+static int parse_tiles(const u8* in, u64 n, u64 hdr, u32 claimed, u32 pshift, bool clean_cuts, Parse& P, bool* complete_out,
+                       u32* tvalid_out) {
     const u32 nfrag = (u32)(((u64)claimed + kBlockSize - 1) / kBlockSize);
-    DecodeResult res{};
-    if (nfrag == 0 || n <= hdr) {  // :1030 -> whole-stream serial decoder (:1154-1155)
-        *path = 3;
-        SerialArgs a{in, n, hdr, out, claimed, &res};
-        as_warp(0, 0, 32);
-        cpu_warp::run_warp(entry_serial, &a);
-        return res.status;
-    }
-    Parse P;
     parse_stream(in, n, hdr, claimed, pshift, P);
     std::vector<u64>& idx = P.idx;
     std::vector<u64>& ost = P.ost;
@@ -219,9 +221,7 @@ static int decode_parsed(const u8* in, u64 n, u64 hdr, u32 claimed, u8* out, u32
     ParseArrays& pa = P.pa;
     const u32 nchunk = P.nchunk, pgrid = (nchunk + kParseThreads - 1) / kParseThreads;
     const u64 pflags = P.pflags, total = P.total, first_err = P.first_err;
-    std::vector<u8> tf(nfrag + 64, 0);
-    // ---- the parse's verdicts (:1049-1058)
-    *path = 1;
+    // ---- the parse's verdicts
     if (first_err != ~0ull) return (int)(first_err & 7);
     if (!(pflags & (PF_ANOMALY | PF_BROKEN)) && total != claimed) return ST_INVALID_INPUT;
     ost[nfrag] = claimed;
@@ -238,7 +238,30 @@ static int decode_parsed(const u8* in, u64 n, u64 hdr, u32 claimed, u8* out, u32
                                    (const u64*)out_off.data(), (const u64*)sfx.data(), n, pshift, nfrag, idx.data(), ost.data());
         k_cut_fill(nfrag, idx.data(), ost.data());
     }
-    const u32 tvalid = complete ? nfrag : tiles_valid(idx, nfrag, n);  // :1083-1095
+    *complete_out = complete;
+    *tvalid_out = complete ? nfrag : tiles_valid(idx, nfrag, n);
+    return 0;
+}
+
+static int decode_parsed(const u8* in, u64 n, u64 hdr, u32 claimed, u8* out, u32 pshift, bool clean_cuts, int* path) {
+    const u32 nfrag = (u32)(((u64)claimed + kBlockSize - 1) / kBlockSize);
+    DecodeResult res{};
+    if (nfrag == 0 || n <= hdr) {  // :1030 -> whole-stream serial decoder (:1154-1155)
+        *path = 3;
+        SerialArgs a{in, n, hdr, out, claimed, &res};
+        as_warp(0, 0, 32);
+        cpu_warp::run_warp(entry_serial, &a);
+        return res.status;
+    }
+    Parse P;
+    bool complete = false;
+    u32 tvalid = 0;
+    *path = 1;
+    const int verdict = parse_tiles(in, n, hdr, claimed, pshift, clean_cuts, P, &complete, &tvalid);
+    if (verdict) return verdict;
+    std::vector<u64>& idx = P.idx;
+    std::vector<u64>& ost = P.ost;
+    std::vector<u8> tf(nfrag + 64, 0);
     // ---- the tiles (:1096-1111)
     if (tvalid) {
         FragArgs a{in, idx.data(), nfrag, tvalid, hdr, n, out, claimed, &res, ost.data(), tf.data()};
@@ -303,6 +326,109 @@ static int validate(const u8* in, u64 n, u64 hdr, u32 claimed, const std::vector
     return res.status;
 }
 
+struct RangeArgs {
+    const RangeDesc* descs;
+    u32 ndesc, nwork;
+    u32* next_work;
+    u8* slots;
+    u64 slot_stride;
+    u32* flags;
+    DecodeResult* res;
+};
+static void entry_range(void* p) {
+    const RangeArgs& a = *(const RangeArgs*)p;
+    k_decode_range(a.descs, a.ndesc, a.nwork, a.next_work, a.slots, a.slot_stride, a.flags, a.res);
+}
+
+// range_launch (snappy_b200.cu) for one request: every warp of the persistent grid in turn (the first one takes every
+// work item); true when every tile was clean.  The slot sits between sentinels that must survive.
+static bool range_launch(const RangeDesc& d, u32 nwork, u64 slot_bytes, bool* slot_guard_ok) {
+    std::vector<u8> slot(slot_bytes + 2 * kGuard + 64, kSentinel);
+    u32 next_work = 0, flag = 0;
+    DecodeResult res{};
+    RangeArgs a{&d, 1u, nwork, &next_work, slot.data() + kGuard, 0, &flag, &res};
+    const u32 warps = nwork < 4 ? nwork : 4;
+    for (u32 w = 0; w < warps; w++) {
+        as_warp(w / kDecodeWarpsPerCta, (w % kDecodeWarpsPerCta) * 32, kDecodeWarpsPerCta * 32);
+        cpu_warp::run_warp(entry_range, &a);
+    }
+    *slot_guard_ok = *slot_guard_ok && sentinels_intact(slot.data(), kGuard) &&
+                     sentinels_intact(slot.data() + kGuard + slot_bytes, kGuard);
+    return !res.fallback && !flag;
+}
+
+// range_chain_locked (snappy_b200.cu) after the header and range checks: path 0 (side index), 1 (the parse's verdict,
+// or its tiles over the range), 2 / 3 (validation, then the whole decode of a valid stream and the copy)
+static int range_chain(const u8* in, u64 n, u64 hdr, u32 claimed, const std::vector<u64>* index, u64 offset, u64 length,
+                       u8* out, u32 pshift, int* path, bool* slot_guard_ok) {
+    const u32 nfrag = (u32)(((u64)claimed + kBlockSize - 1) / kBlockSize);
+    const u64 end = offset + length;
+    RangeDesc d{};
+    d.in = in;
+    d.out = out;
+    d.in_begin = hdr;
+    d.in_end = n;
+    d.out_len = claimed;
+    d.offset = offset;
+    d.length = length;
+    d.nfrag = nfrag;
+    bool valid = false;
+    if (index) {  // range_indexed_locked
+        *path = 0;
+        if (length == 0) return ST_OK;
+        d.frag_off = index->data();
+        d.t0 = (u32)(offset / kBlockSize);
+        const u32 t1 = (u32)((end - 1) / kBlockSize);
+        const u64 ob = (u64)d.t0 * kBlockSize, oe = ob + kBlockSize < end ? ob + kBlockSize : end;
+        if (range_launch(d, t1 - d.t0 + 1, ob < offset ? oe - ob : 0, slot_guard_ok)) return ST_OK;
+    }
+    Parse P;
+    if (nfrag > 0 && n > hdr) {  // range_parsed_locked
+        bool complete = false;
+        u32 tvalid = 0;
+        *path = 1;
+        const int verdict = parse_tiles(in, n, hdr, claimed, pshift, true, P, &complete, &tvalid);
+        if (verdict) return verdict;
+        if (complete) {
+            valid = true;
+            if (length == 0) return ST_OK;
+            u64 t3[3];
+            launch_independent_threads(1u, 1u, k_range_tiles, (const u64*)P.ost.data(), nfrag, offset, end, t3);
+            d.frag_off = P.idx.data();
+            d.out_start = P.ost.data();
+            d.t0 = (u32)t3[0];
+            if (range_launch(d, (u32)t3[1] - d.t0 + 1, t3[2], slot_guard_ok)) return ST_OK;
+        }
+    }
+    // range_whole_locked
+    int st = ST_OK, vpath = 3;
+    if (!valid) {
+        bool step3 = false;
+        st = validate(in, n, hdr, claimed, nullptr, pshift, &vpath, &step3);
+    }
+    if (st == ST_OK) {
+        std::vector<u8> whole((size_t)claimed + 64);
+        st = decode_parsed(in, n, hdr, claimed, whole.data(), pshift, true, &vpath);
+        if (st == ST_OK && length) memcpy(out, whole.data() + offset, length);
+    }
+    *path = vpath == 3 ? 3 : 2;
+    return st;
+}
+
+// CRC-32 (zlib's), so that the test can compare bytes without writing them out
+static u32 crc32(const u8* p, size_t n) {
+    static u32 table[256];
+    if (!table[1])
+        for (u32 i = 0; i < 256; i++) {
+            u32 c = i;
+            for (int k = 0; k < 8; k++) c = (c & 1) ? 0xEDB88320u ^ (c >> 1) : c >> 1;
+            table[i] = c;
+        }
+    u32 c = 0xffffffffu;
+    for (size_t i = 0; i < n; i++) c = table[(c ^ p[i]) & 0xff] ^ (c >> 8);
+    return c ^ 0xffffffffu;
+}
+
 // the oracle's status of uncompress (sjo_uncompress_ex into a buffer of the claimed length)
 static int oracle_status(const u8* s, size_t n) {
     u32 claimed = 0;
@@ -327,12 +453,6 @@ static std::vector<u8> slurp(const char* path) {
     if (sz && fread(b.data(), 1, sz, fp) != sz) exit(2);
     fclose(fp);
     return b;
-}
-
-static bool sentinels_intact(const u8* p, size_t len) {
-    for (size_t i = 0; i < len; i++)
-        if (p[i] != kSentinel) return false;
-    return true;
 }
 
 static int run_parsed(int argc, char** argv) {
@@ -535,12 +655,64 @@ static int run_validate_pages(int argc, char** argv) {
     return failed ? 1 : 0;
 }
 
+// mode "range": uncompress_range_locked for every range of F.ranges (text, "offset length" per line), with the side index
+// F<IDX_SUFFIX> when that file exists.  The output lies between sentinels.  Per range: the status, the path, the CRC-32
+// of the bytes on OK and whether every sentinel (around the output and the scratch slot) survived.
+static int run_range(int argc, char** argv) {
+    const u32 pshift = getenv("PSHIFT") ? (u32)atoi(getenv("PSHIFT")) : kParseChunkLog2;
+    const char* suffix = getenv("IDX_SUFFIX");
+    for (int ai = 2; ai < argc; ai++) {
+        std::vector<u8> s = slurp(argv[ai]);
+        const size_t sz = s.size();
+        u8* in = (u8*)aligned_alloc(256, (sz + 64 + 255) & ~(size_t)255);
+        memset(in, 0, sz + 64);
+        if (sz) memcpy(in, s.data(), sz);
+        std::vector<u64> index;
+        bool have_index = false;
+        if (suffix) {
+            const std::string ip = std::string(argv[ai]) + suffix;
+            if (FILE* fp = fopen(ip.c_str(), "rb")) {
+                fclose(fp);
+                std::vector<u8> raw = slurp(ip.c_str());
+                index.resize(raw.size() / 8);
+                memcpy(index.data(), raw.data(), index.size() * 8);
+                have_index = true;
+            }
+        }
+        FILE* rf = fopen((std::string(argv[ai]) + ".ranges").c_str(), "r");
+        if (!rf) exit(2);
+        unsigned long long offset, length;
+        while (fscanf(rf, "%llu %llu", &offset, &length) == 2) {
+            u32 claimed = 0;
+            size_t hdr = 0;
+            int st = sjo_parse32(in, sz, 0, &claimed, &hdr), path = -1;
+            bool slot_ok = true;
+            std::vector<u8> buf(length + 2 * kGuard, kSentinel);
+            u8* out = buf.data() + kGuard;
+            if (st == ST_OK && (offset > claimed || length > claimed - offset)) st = 10;  // SNAPPY_B200_BAD_ARGUMENT
+            else if (st == ST_OK)
+                st = range_chain(in, sz, hdr, claimed, have_index ? &index : nullptr, offset, length, out, pshift, &path,
+                                 &slot_ok);
+            const bool guard_ok = slot_ok && sentinels_intact(buf.data(), kGuard) && sentinels_intact(out + length, kGuard);
+            char ps[8];
+            if (path < 0) snprintf(ps, sizeof ps, "-");
+            else snprintf(ps, sizeof ps, "%d", path);
+            printf("%s: range %llu+%llu status %d path %s crc %08x guard %s\n", argv[ai], offset, length, st, ps,
+                   st == ST_OK ? crc32(out, length) : 0u, guard_ok ? "ok" : "CHANGED");
+        }
+        fclose(rf);
+        free(in);
+    }
+    return 0;
+}
+
 int main(int argc, char** argv) {
     if (argc < 2) return 2;
     if (!strcmp(argv[1], "parsed")) return run_parsed(argc, argv);
     if (!strcmp(argv[1], "pages")) return run_pages(argc, argv);
     if (!strcmp(argv[1], "validate")) return run_validate(argc, argv);
     if (!strcmp(argv[1], "validate-pages")) return run_validate_pages(argc, argv);
-    fprintf(stderr, "mode: parsed | pages | validate | validate-pages\n");
+    if (!strcmp(argv[1], "range")) return run_range(argc, argv);
+    fprintf(stderr, "mode: parsed | pages | validate | validate-pages | range\n");
     return 2;
 }
